@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the niwqg ETDRK4 hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Metric (BASELINE.json): fp64 grid-point-steps/s of the coupled NIW-QG model.
 Default workload: CoupledModel, Lamb dipole + uniform NIW, 8192^2, fp64, exponential filter on
@@ -156,6 +156,32 @@ class ClockSampler(object):
         return out
 
 
+DUMP_MAX_POINTS = 1 << 21     # q (8 B) + phi (16 B) per point: a dump stays under 48 MB at any grid size
+
+
+def dump_outputs(out_dir, h, qg, suffix=""):
+    """Write what the timed steps computed, as a caller of the stepping path receives it, to out_dir/<name><suffix>.npy:
+    the physical fields q and phi of every member (phi as float64 with a last axis of (real, imag)) and the integrated
+    budgets Ke, Pw, Kw per member.  Fields of more than DUMP_MAX_POINTS points are sampled at fixed points (seeded, the
+    same in every run and build), so two builds run with the same arguments can be compared output for output."""
+    from niwqg_b200 import _native as nat
+    q = h.field("Q")
+    phi = None if qg else h.field("PHI")
+    if q.size > DUMP_MAX_POINTS:
+        idx = np.unique(np.random.RandomState(0).randint(0, q.size, DUMP_MAX_POINTS))
+        q = q.reshape(-1)[idx]
+        phi = None if qg else phi.reshape(-1)[idx]
+    out = {"q": q}
+    if not qg:
+        out["phi"] = np.stack([phi.real, phi.imag], axis=-1)
+    sc = h.scalars()
+    for name, slot in (("Ke", "KE"),) if qg else (("Ke", "KE"), ("Pw", "PW"), ("Kw", "KW")):
+        out[name] = sc[:, nat.S[slot]]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def slab_parity(dist, local, rank, world):
     """N > 1: the slab-decomposed run against the single-GPU run of the same model (rank 0 holds both).
     (1) 2048^2, 3 steps from a perturbed Lamb dipole: q, phi, qh, Ke;  (2) 8192^2, 2 steps from the bench initial condition
@@ -286,6 +312,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = world * npts * args.steps / (ms * 1e-3)     # slab: world * (nx^2 / world) = the one grid
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, h, qg, "_rank%d" % rank if world > 1 else "")
 
     # ---------------- per-kernel-kind timing (separate short run with events around every launch)
     nprof = min(args.steps, 3)
@@ -576,7 +604,14 @@ def main():
                     help="N > 1: slab-decompose the one grid (strong scaling, default) or one member per GPU (weak)")
     ap.add_argument("--no-ensemble", action="store_true", help="N > 1 slab run: skip the extra ensemble_weak measurement")
     ap.add_argument("--no-check", action="store_true", help="N > 1 slab run: skip the parity leg (slab vs single GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write q, phi (a fixed sample of points on large grids) and the budgets "
+                         "Ke, Pw, Kw as DIR/<name>.npy (float64; _rank<r> appended with N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

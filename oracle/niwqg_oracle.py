@@ -15,15 +15,14 @@ that feeds back into the step.  It is organised differently from the reference
 generation so 4096^2+ initialises in bounded memory), but every floating point
 operation is issued in the same order as the reference issues it, so results
 are bit-identical to the reference on the same numpy.  Each method cites the
-reference lines it follows (paths relative to /root/reference).
+reference lines it follows (paths relative to the reference checkout).
 
 Pinning
 -------
 Parity is PINNED: ``tests/golden/make_golden.py`` imports the unmodified
-reference from /root/reference (with an ``h5py`` import stub) in the build
-container and stores its outputs under ``tests/golden/*.npz``;
-``tests/test_oracle_cpu.py`` checks this oracle against those vectors
-bit-for-bit, and (when /root/reference is present) against the live reference.
+reference from a checkout of it (with an ``h5py`` import stub) and stores its
+outputs under ``tests/golden/*.npz``; ``tests/test_oracle_cpu.py`` checks this
+oracle against those vectors bit-for-bit.
 
 Third-party arithmetic the reference relies on: ``numpy.fft`` (pocketfft,
 numpy>=1.8 per requirements.txt:1, 2.3.5 installed) - called here through the

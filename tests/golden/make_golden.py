@@ -1,8 +1,7 @@
-"""Generate golden vectors from the UNMODIFIED reference at /root/reference.
+"""Generate golden vectors from the UNMODIFIED reference (a checkout of the niwqg project; the
+directory that holds its ``niwqg`` package):
 
-Run in the build container only (the reference does not travel to the GPU box):
-
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py REFERENCE_DIR [CASE ...]
 
 The reference imports ``h5py`` at module top (niwqg/Kernel.py:4) but only
 dereferences it when save_to_disk=True; h5py is not installed here, so a stub
@@ -15,14 +14,14 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def import_reference():
+def import_reference(ref_dir):
     if "h5py" not in sys.modules:
         try:
             import h5py  # noqa: F401
         except Exception:
             sys.modules["h5py"] = types.ModuleType("h5py")
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
+    if ref_dir not in sys.path:
+        sys.path.insert(0, ref_dir)
     import logging
     import niwqg
     from niwqg import CoupledModel, UnCoupledModel, YBJModel, QGModel, InitialConditions
@@ -161,8 +160,10 @@ def reference_tests_known_answers(ctor):
 
 
 if __name__ == "__main__":
-    ctor, ic = import_reference()
-    only = sys.argv[1:]          # optional: regenerate just these cases
+    if len(sys.argv) < 2:
+        raise SystemExit(__doc__)
+    ctor, ic = import_reference(os.path.abspath(sys.argv[1]))
+    only = sys.argv[2:]          # optional: regenerate just these cases
     for case in CASES:
         if not only or case[0] in only:
             run_case(ctor, ic, *case)
