@@ -413,8 +413,9 @@ __device__ __forceinline__ cd etd_update(int stage, cd y0, cd y1, cd Fn, cd& F0,
 }
 
 // ST (stage 1..4), DQ / DP (update the q / phi equation) are compile-time so that every instantiation carries only
-// the loads of its stage and equation: the fused (DQ && DP) body needs 128 registers and runs at ~79 % of the HBM
-// peak, the two halves launched back to back are lighter and faster (they share only the 8 B filter value).
+// the loads of its stage and equation.  Every launch updates one equation: a body that updated both needed 128 registers
+// and ran at ~79 % of the HBM peak, the two halves launched back to back are lighter and faster (they share only the 8 B
+// filter value).
 template <int ST, bool DQ, bool DP>
 __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
     const int N = a.g.N, H = N >> 1, NC = a.g.ncl;

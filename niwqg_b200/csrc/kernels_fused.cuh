@@ -87,20 +87,6 @@ __device__ __forceinline__ void fused_combine(const cd* __restrict__ T, const cd
     for (int p = 0; p < 16; ++p) u[fftc::outidx<16>(p)] = v[p];
 }
 
-// L2 prefetch of the column transforms the NEXT work unit of this CTA will combine (16 lines per thread): issued before
-// the long register-only phases of the current unit, so that the next fused_combine finds its operands in L2
-template <int N>
-__device__ __forceinline__ void fused_prefetch_next(const cd* __restrict__ T, const cd* __restrict__ twc, int unit, int tid) {
-    using G = FusedGeom<N>;
-    if (unit >= G::UNITS) return;
-    FusedThread t;
-    fused_thread<N>(unit, tid, twc, t);
-    if (tid & 7) return;                         // one request per 128 B line (8 consecutive columns)
-    constexpr int M = N / 16;
-#pragma unroll
-    for (int r = 0; r < 16; ++r) prefetch_l2(&T[(size_t)(r * M + t.fam) * N + t.col]);
-}
-
 // inverse radix stage (decimation in frequency, see k_split_p<DIF>) of the 16 spectral values v[r] = s[fam + M r][col]:
 // prologue, conj, x butterfly, radix 16, twiddles; stored as row q M + fam of `out`
 template <int N>
@@ -140,7 +126,6 @@ struct FStageArgs {
     const cd* T;       // M-point column transforms (block layout) of the forward transform this kernel consumes
     cd* out[3];        // k_fstage_phi: radix-stage intermediates of phi, phix, phiy
     int nout;
-    int pf_next;       // L2 prefetch of the next unit's column transforms
     const cd* twc;
     double dk;
 };
@@ -163,25 +148,8 @@ __device__ __forceinline__ void eq_load(EqIn& in, const cd* __restrict__ y0, con
     else { in.c0 = __ldg(&t.E[i]); in.c1 = __ldg(&t.f0[i]); in.c2 = __ldg(&t.fab[i]); in.c3 = __ldg(&t.fc[i]); }
     in.fl = __ldg(&filtr[i]);
 }
-// L2 prefetch of the same operands a few elements ahead: costs no registers, and turns the HBM latency of the register
-// loads into an L2 hit (at 512 threads per SM the two elements in flight per thread cannot cover HBM latency alone)
-template <int ST, bool PHI>
-__device__ __forceinline__ void eq_prefetch(const cd* y0, const cd* y, const cd* y1, const cd* F0, const cd* Fab, const TableSet& t,
-                                            const double* filtr, size_t i) {
-    prefetch_l2(&y0[i]);
-    if (PHI && ST >= 2) prefetch_l2(&y[i]);
-    if (ST >= 3) { prefetch_l2(&F0[i]); prefetch_l2(&Fab[i]); }
-    if (ST == 3) prefetch_l2(&y1[i]);
-    if (ST <= 3) { prefetch_l2(&t.E2[i]); prefetch_l2(&t.Q[i]); }
-    else { prefetch_l2(&t.E[i]); prefetch_l2(&t.f0[i]); prefetch_l2(&t.fab[i]); prefetch_l2(&t.fc[i]); }
-    if ((threadIdx.x & 1) == 0) prefetch_l2(&filtr[i]);
-}
-constexpr int FUSED_PD = 0;     // L2 prefetch distance in elements (0 = off: measured slower, 24.1 vs 22.2 ms of spectral kernels per step)
 // register pipeline depth of the element loop per stage: as deep as 128 registers allow
-#ifndef NIWQG_DEPTH_BOOST
-#define NIWQG_DEPTH_BOOST 0
-#endif
-template <int ST> struct FusedDepth { static constexpr int Q = (ST <= 2 ? 4 : 3) + NIWQG_DEPTH_BOOST, PHI = (ST <= 2 ? 4 : (ST == 3 ? 3 : 2)) + NIWQG_DEPTH_BOOST, INV = 6; };
+template <int ST> struct FusedDepth { static constexpr int Q = ST <= 2 ? 4 : 3, PHI = ST <= 2 ? 4 : (ST == 3 ? 3 : 2), INV = 6; };
 // etd_update (kernels_family.cuh) on preloaded operands; F0 / Fab come back as what the stage stores
 template <int ST>
 __device__ __forceinline__ cd eq_update(const EqIn& in, cd y0, cd Fn, cd& F0, cd& Fab) {
@@ -218,7 +186,6 @@ __global__ void __launch_bounds__(256, 2) k_fstage_q(FStageArgs a) {
 #pragma unroll
             for (int q = 0; q < 16; ++q) xs[q * 256 + tid] = u[q];      // parked: own value and the partner's come from here
         }
-        if (a.pf_next) fused_prefetch_next<N>(a.T, a.twc, unit + gridDim.x, tid);
         __syncthreads();
         const double k1 = a.dk * (double)sidx(t.col, N);
         const size_t i0 = (size_t)t.fam * N + t.col;
@@ -308,7 +275,9 @@ __global__ void __launch_bounds__(256, 2) k_fstage_phi(FStageArgs a) {
 #pragma unroll
             for (int q = 0; q < 16; ++q) xs[q * 256 + tid] = u[q];      // parked (only this thread reads them back)
         }
-        if (a.pf_next) fused_prefetch_next<N>(a.T, a.twc, unit + gridDim.x, tid);
+        // no data dependence (only this thread reads xs back): a scheduling boundary, so that the operand loads below are
+        // not hoisted into the combine, where the 16 values are still live (that spills past 128 registers)
+        __syncwarp();
         const double k1 = a.dk * (double)sidx(t.col, N);
         const size_t i0 = (size_t)t.fam * N + t.col;
         double s[SE_COUNT];
@@ -366,7 +335,6 @@ struct FInvertArgs {
     InvertArgs i;
     const cd* T;       // M-point column transforms (block layout) of fft(|phi|^2 + i J): MF_WAVE_PV only
     cd *out_uv, *out_qs;
-    int pf_next;
     const cd* twc;
     double dk;
 };
@@ -392,7 +360,6 @@ __global__ void __launch_bounds__(256, 2) k_finvert(FInvertArgs a) {
             fused_combine<N>(a.T, a.twc, t, u);
 #pragma unroll
             for (int q = 0; q < 16; ++q) xs[q * 256 + tid] = u[q];
-            if (a.pf_next) fused_prefetch_next<N>(a.T, a.twc, unit + gridDim.x, tid);
             __syncthreads();
         }
         cd u[16];

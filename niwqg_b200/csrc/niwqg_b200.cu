@@ -88,21 +88,18 @@ struct niwqg_handle {
     cudaStream_t lane_stream[NLANE] = {nullptr, nullptr};
     ncclComm_t lane_comm[NLANE] = {nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    bool lanes = false;         // second lane usable
     // CUDA graphs of one whole step, one per ping-pong parity of the state buffers (key = cq*4 + cp*2 + cc): small grids
     // are launch-bound (~100 launches of a few microseconds each per step)
     struct StepGraph { cudaGraphExec_t exec = nullptr; int cq = 0, cp = 0, cc = 0; long long launches = 0; };
     StepGraph graphs[8];
     bool use_graphs = false;
     int direct_steps = 0;       // steps issued without a graph (the first ones set kernel attributes lazily)
-    bool in_group = false;      // inside fft2_group with both lanes active
-    int group_occ_limit = 0;    // 1: passes of a two-lane group run one CTA per SM (measured slower: off)
     int exchange = 0;           // 0: pushes fused into the first pass; 1: first pass writes the exchange layout locally,
                                 // the copy engines move the chunks to the peers (no SM involved, overlaps the other lane)
     cd* Xl[NLANE] = {nullptr, nullptr};   // per-lane send staging of the copy-engine exchange
     ncclComm_t comm = nullptr;
-    int col3 = 1;               // 8192^2, one GPU: three-pass column transform (0.714 vs 0.771 ms for the cluster kernel);
-                                // NIWQG_COL3=0 switches back
+    bool col3 = false;          // 8192^2, one GPU, one member, not split: three-pass column transform (0.714 vs 0.771 ms
+                                // for the cluster kernel)
     cd* S3[2] = {nullptr, nullptr};   // its scratch array, one per lane
     cd* tw_c3 = nullptr;              // stage twiddles of its 512-point local transforms
     // split transforms (fft_split.cuh): x = 2 x N/2 on de-interleaved physical rows, y = 16 x N/16, three streaming launches
@@ -125,24 +122,10 @@ struct niwqg_handle {
     void* stage_out[2] = {nullptr, nullptr};  // one member: real (npts * 8) / complex (npts * 16)
     double* pin = nullptr;                    // pinned host scratch for the scalars of diagnostics / status
     int slab_panel = 0;         // slab, pushed exchange of inverse transforms: panel receive layout (FftArgs::panel); = cluster
-                                // size of the column pass for N >= 1024 (NIWQG_SLAB_PANEL=0 keeps rows of ncl columns)
+                                // size of the column pass for N >= 1024, else 0 (rows of ncl columns)
     int flag_barrier = 1;       // slab: peer-memory flags instead of the 1-element all-reduce between the two passes
                                 // (validated on 2 and 8 GPUs: 13.33 vs 13.47 ms/step at 8; NIWQG_SLAB_BARRIER=nccl switches back)
     unsigned bar_epoch[NLANE] = {0, 0};
-    int row_bulk = 1;           // split path: row tiles fetched by one bulk copy (cp.async.bulk; NIWQG_ROW_BULK=0: 16 LDG.128 per thread)
-    int fused = 1;              // split path, Coupled / UnCoupled: spectral kernels fused with the radix stage (kernels_fused.cuh);
-                                // NIWQG_FUSED=0 runs the stage as launches of its own
-    int row_loader = 3;         // split path: physical products formed by the forward row passes' loaders: bit 0 wave-PV pair,
-                                // bit 1 (uq, vq)  (NIWQG_ROW_LOADER=0: pointwise kernels)
-    int hsym = 1;               // q-equation stage kernels update one element of every (K, -K) pair and store both (NIWQG_HSYM=0: every element)
-    int fused_pf = 0;           // fused kernels prefetch the next unit's operands into L2 (NIWQG_FUSED_PF=1)
-    int fused_grid = 296;       // persistent grid of the fused kernels: 2 CTAs per SM
-    int split_stage = 1;        // k_spec_stage as two lighter launches (q equation / phi equation): NIWQG_SPLIT_STAGE=0 fuses
-    int tma = 1;                // column passes whose rows are narrower than a 128 B line fetch their tile by TMA
-                                // (1024^2: 4345 -> 4983 GB/s); NIWQG_TMA=0 switches it off
-    int fft_variant = 6;        // FftArgs::variant: column clusters push (DIF, plain remote stores), row clusters pull (DIT):
-                                // measured best (profiles/r01b_cluster_variants.txt, r01d_async_push.txt)
-    int pf_ctas = 296;          // L2 prefetch distance of the FFT passes in CTAs (~ one resident wave: 148 SMs x 2)
     // optional per-kernel-kind CUDA-event timing (bench.py's roofline leg)
     bool prof = false;
     struct ProfRec { int kind; cudaEvent_t a, b; };
@@ -281,16 +264,22 @@ __global__ void k_slab_wait(const unsigned* flags, int nranks, unsigned epoch) {
     } while (v < epoch);
 }
 
+// one resident wave of the FFT passes and of the persistent fused kernels: 148 SMs x 2 CTAs
+static constexpr int WAVE_CTAS = 296;
+
 static void fft_common_args(niwqg_handle* h, FftArgs& a) {
     a.twc = h->twc;
     a.dk = h->dk;
-    a.pf_groups = h->pf_ctas;
-    a.variant = h->fft_variant;
+    a.pf_groups = WAVE_CTAS;    // L2 prefetch distance of the FFT passes in CTAs
+    // variant and one_cta_per_sm are constants on the host: column clusters push (DIF, plain remote stores), row clusters
+    // pull (DIT), two CTAs per SM (measured best: profiles/r01b_cluster_variants.txt, r01d_async_push.txt)
+    a.variant = 6;
+    a.one_cta_per_sm = 0;
     a.g = h->g;
     a.xmap_in = a.xmap_out = 0;
     a.deint_in = a.deint_out = 0;
-    a.one_cta_per_sm = 0;
-    a.tma_in = h->tma;
+    a.tma_in = 1;               // column passes whose rows are narrower than a 128 B line fetch their tile by TMA
+                                // (1024^2: 4345 -> 4983 GB/s)
     a.xchunk = h->nyl * h->ncl;
     a.mstride = h->npts;
     a.pitch = h->ncl;
@@ -304,7 +293,7 @@ static int split_rows(niwqg_handle* h, const void* in, void* out, int pro, int e
     a.in = in; a.out = out; a.pro = pro; a.epi = epi; a.tw = h->tw_half;
     a.nlines = 2 * h->N; a.pitch = Nh; a.mstride = (size_t)Nh * Nh; a.g = Grid{Nh, h->dk, Nh, Nh / 2, 0, 0};
     a.conj_in = 0; a.conj_out = conj_out ? 1 : 0; a.scale = sc; a.scale_im = conj_out ? -sc : sc;
-    a.tma_in = h->row_bulk ? 2 : 0;
+    a.tma_in = 2;          // row tiles fetched by one bulk copy (cp.async.bulk) instead of 16 LDG.128 per thread
     a.pf_groups = 0;       // measured on 16384 lines of 4096: 0.362 ms without the L2 prefetch, 0.382 ms with it
     { PROF(PK_FFT_ROW); CK(launch_pass<false>(Nh, a, 1, h->stream)); }
     h->launches++;
@@ -312,7 +301,7 @@ static int split_rows(niwqg_handle* h, const void* in, void* out, int pro, int e
 }
 // forward row pass that forms its input while loading the operands: LD_WAVEPV W = |phi|^2 + i jscale i J(phi*,phi) from phi,
 // phix, phiy (replaces k_phys_wavepv and the re-read of W), LD_UQVQ P1 = (uq, vq) from uv, qs (k_phys_rhs then skips the P1
-// store); NIWQG_ROW_LOADER=0 keeps the pointwise kernels
+// store)
 static int split_rows_loader(niwqg_handle* h, int ld, cd* out) {
     FftArgs a{};
     fft_common_args(h, a);
@@ -407,9 +396,7 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
         // pass 1: rows
         a.in = in; a.out = out; a.pro = pro; a.epi = EPI_NONE; a.tw = h->tw_row; a.nlines = h->N;
         a.conj_in = inverse ? 1 : 0; a.conj_out = 0; a.scale = 1.0; a.scale_im = 1.0;
-        a.deint_in = (!inverse && h->deintC > 1); a.deint_out = (inverse && h->deintC > 1);   // the x side of the row pass
         { PROF_ON(PK_FFT_ROW, lane); CK(launch_pass<false>(h->N, a, batch, h->lane_stream[lane])); }
-        a.deint_in = a.deint_out = 0;
         // pass 2: columns
         a.in = out; a.out = final_out; a.pro = PRO_NONE; a.epi = epi; a.tw = h->tw_col; a.nlines = h->N;
         a.conj_in = 0; a.conj_out = inverse ? 1 : 0;
@@ -421,7 +408,6 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
     if (batch != 1) { h->err = "slab transforms take one member"; return -1; }
     if (h->p2p) {
         cudaStream_t st = h->lane_stream[lane];
-        a.one_cta_per_sm = h->in_group ? h->group_occ_limit : 0;
         // fused exchange: the first pass stores into the owners' receive buffers over NVLink; one tiny all-reduce is
         // the barrier that says "everybody's pushes have landed"; the second pass reads the local receive buffer.
         const int b = h->ybuf[lane];
@@ -436,9 +422,9 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
         a.in = in; a.out = ce ? (void*)h->Xl[lane] : nullptr; a.pro = pro; a.epi = EPI_NONE; a.scale = 1.0; a.scale_im = 1.0;
         a.conj_out = 0;
         if (!inverse) {
-            a.tw = h->tw_row; a.nlines = h->nyl; a.conj_in = 0; a.deint_in = (h->deintC > 1); a.xmap_out = ce ? 1 : 0;
+            a.tw = h->tw_row; a.nlines = h->nyl; a.conj_in = 0; a.xmap_out = ce ? 1 : 0;
             { PROF_ON(PK_FFT_ROW, lane); CK(launch_pass<false>(h->N, a, 1, st)); }
-            a.deint_in = 0; a.xmap_out = 0;
+            a.xmap_out = 0;
         } else {
             a.tw = h->tw_col; a.nlines = h->ncl; a.conj_in = 1;
             { PROF_ON(PK_FFT_COL, lane); CK(launch_pass<true>(h->N, a, 1, st)); }
@@ -464,7 +450,6 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
             { PROF_ON(PK_FFT_COL, lane); CK(launch_pass<true>(h->N, a, 1, st)); }
         } else {
             a.tw = h->tw_row; a.nlines = h->nyl; a.xmap_in = 1; a.conj_out = 1; a.scale = sc; a.scale_im = -sc;
-            a.deint_out = (h->deintC > 1);
             { PROF_ON(PK_FFT_ROW, lane); CK(launch_pass<false>(h->N, a, 1, st)); }
         }
         h->launches += 3;
@@ -472,9 +457,8 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
     }
     if (!inverse) {
         a.in = in; a.out = h->X; a.pro = pro; a.epi = EPI_NONE; a.tw = h->tw_row; a.nlines = h->nyl; a.xmap_out = 1;
-        a.conj_in = 0; a.conj_out = 0; a.scale = 1.0; a.scale_im = 1.0; a.deint_in = (h->deintC > 1);
+        a.conj_in = 0; a.conj_out = 0; a.scale = 1.0; a.scale_im = 1.0;
         { PROF(PK_FFT_ROW); CK(launch_pass<false>(h->N, a, 1, h->stream)); }
-        a.deint_in = 0;
         int r = slab_all_to_all(h, h->X, h->Y);
         if (r) return r;
         a.in = h->Y; a.out = final_out; a.pro = PRO_NONE; a.epi = epi; a.tw = h->tw_col; a.nlines = h->ncl; a.xmap_out = 0;
@@ -486,17 +470,15 @@ static int fft2(niwqg_handle* h, const void* in, cd* out, bool inverse, int pro,
         int r = slab_all_to_all(h, h->X, h->Y);
         if (r) return r;
         a.in = h->Y; a.out = final_out; a.pro = PRO_NONE; a.epi = epi; a.tw = h->tw_row; a.nlines = h->nyl; a.xmap_in = 1;
-        a.deint_out = (h->deintC > 1);
         a.conj_in = 0; a.conj_out = 1; a.scale = sc; a.scale_im = -sc;
         { PROF(PK_FFT_ROW); CK(launch_pass<false>(h->N, a, 1, h->stream)); }
     }
     h->launches += 2;
     return 0;
 }
-// column pass of the natural layout: the cluster kernel, or - 8192^2 with NIWQG_COL3 - the three-pass variant
+// column pass of the natural layout: the cluster kernel, or - 8192^2, see niwqg_handle::col3 - the three-pass variant
 static cudaError_t launch_col_natural(niwqg_handle* h, const FftArgs& a, int batch, int lane) {
-    if (h->col3 && h->N == 8192 && batch == 1 && a.epi == EPI_NONE)
-    {
+    if (h->col3 && a.epi == EPI_NONE) {
         FftArgs b = a;
         b.tw = h->tw_c3;
         h->launches++;      // two kernels for this pass (the caller counts one)
@@ -511,7 +493,6 @@ static int inv_row_pass(niwqg_handle* h, const cd* in, cd* out, int pro, int lan
     fft_common_args(h, a);
     a.in = in; a.out = out; a.pro = pro; a.epi = EPI_NONE; a.tw = h->tw_row; a.nlines = h->N;
     a.conj_in = 1; a.conj_out = 0; a.scale = 1.0; a.scale_im = 1.0;
-    a.deint_out = (h->deintC > 1);
     { PROF_ON(PK_FFT_ROW, lane); CK(launch_pass<false>(h->N, a, h->B, h->lane_stream[lane])); }
     h->launches++;
     return 0;
@@ -560,7 +541,6 @@ static int slab_inv_row(niwqg_handle* h, int lane, int b, cd* out, int pro) {
     a.nyl_shift = sh;
     a.panel = h->slab_panel;
     a.tw = h->tw_row; a.nlines = h->nyl; a.xmap_in = 1; a.conj_out = 1; a.scale = sc; a.scale_im = -sc;
-    a.deint_out = (h->deintC > 1);
     { PROF_ON(PK_FFT_ROW, lane); CK(launch_pass<false>(h->N, a, 1, h->lane_stream[lane])); }
     h->launches++;
     return 0;
@@ -591,19 +571,14 @@ static int slab_barrier(niwqg_handle* h, int lane, cudaStream_t st) {
 struct FftJob { const void* in; cd* out; bool inverse; int pro; };
 static int fft2_group(niwqg_handle* h, const FftJob* jobs, int n) {
     // (one GPU: the column pass of one transform, bound by the DSMEM exchange, runs next to the row pass of the other)
-    const bool par = h->lanes && (h->p2p || h->nranks == 1) && !h->prof && n > 1 && !h->split;
+    const bool par = (h->p2p || h->nranks == 1) && !h->prof && n > 1 && !h->split;
     if (!par) {
         for (int i = 0; i < n; ++i) FFT(jobs[i].in, jobs[i].out, jobs[i].inverse, jobs[i].pro, h->B);
         return 0;
     }
     CK(cudaEventRecord(h->ev_fork, h->lane_stream[0]));
     CK(cudaStreamWaitEvent(h->lane_stream[1], h->ev_fork, 0));
-    h->in_group = true;
-    for (int i = 0; i < n; ++i) {
-        int r = fft2(h, jobs[i].in, jobs[i].out, jobs[i].inverse, jobs[i].pro, h->B, EPI_NONE, nullptr, i & 1);
-        if (r) { h->in_group = false; return r; }
-    }
-    h->in_group = false;
+    for (int i = 0; i < n; ++i) FFT(jobs[i].in, jobs[i].out, jobs[i].inverse, jobs[i].pro, h->B, EPI_NONE, nullptr, i & 1);
     CK(cudaEventRecord(h->ev_join, h->lane_stream[1]));
     CK(cudaStreamWaitEvent(h->lane_stream[0], h->ev_join, 0));
     return 0;
@@ -700,7 +675,7 @@ static int wave_fields(niwqg_handle* h, bool want_phi, bool grad, bool lap) {
         // phi = ifft(phih), phix = ifft(ik phih), phiy = ifft(il phih) in 2 row passes + 3 column passes instead of 3 + 3:
         // the i l factor depends on the column-pass direction only, so phiy shares the row pass of phi and gets its
         // factor (conjugated: the intermediate is in the conjugated domain) in the prologue of its column pass.
-        const bool par = h->lanes && !h->prof;
+        const bool par = !h->prof;
         const int l1 = par ? 1 : 0;
         if (par) {
             CK(cudaEventRecord(h->ev_fork, h->lane_stream[0]));
@@ -721,7 +696,7 @@ static int wave_fields(niwqg_handle* h, bool want_phi, bool grad, bool lap) {
     if (h->nranks > 1 && h->p2p && h->exchange == 0 && want_phi && grad && !lap) {
         // slab: the column pass comes first, so phi and phix share it (one exchange less): phix gets its conj(i k) in the
         // prologue of its row pass, phiy = ifft(il phih) has its own column pass
-        const bool par = h->lanes && !h->prof;
+        const bool par = !h->prof;
         const int l1 = par ? 1 : 0;
         if (par) {
             CK(cudaEventRecord(h->ev_fork, h->lane_stream[0]));
@@ -812,16 +787,15 @@ static int step_family_fused_n(niwqg_handle* h) {
     const int oq = h->cq, op = h->cp, nq = 1 - oq, np = 1 - op;
     const bool wave = (h->flags & MF_WAVE_PV) != 0;
     const double sc = 1.0 / ((double)N * (double)N);
-    const int grid = h->fused_grid;
+    const int grid = WAVE_CTAS;     // persistent grid of the fused kernels
     int r;
     for (int st = 1; st <= 4; ++st) {
-        PhysArgs pa = phys_args(h, (h->row_loader & 2) ? MF_P1_BY_LOADER : 0);
+        PhysArgs pa = phys_args(h, MF_P1_BY_LOADER);
         { PROF(PK_PHYS); k_phys_rhs<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(pa); }
         CK(cudaGetLastError());
         h->launches++;
         FIN(SD_COUNT, h->sumsD);
-        if (h->row_loader & 2) { if ((r = split_rows_loader(h, LD_UQVQ, h->P1))) return r; }   // P1 = (uq, vq) formed while loading uv, qs
-        else if ((r = split_rows(h, h->P1, h->P1, PRO_NONE, EPI_NONE, 1.0, false))) return r;
+        if ((r = split_rows_loader(h, LD_UQVQ, h->P1))) return r;   // P1 = (uq, vq) formed while loading uv, qs
         if ((r = split_colsub(h, h->P1, h->T[0], true))) return r;
         if ((r = split_rows(h, h->P2, h->P2, PRO_NONE, EPI_NONE, 1.0, false))) return r;
         if ((r = split_colsub(h, h->P2, h->T[1], true))) return r;
@@ -833,8 +807,8 @@ static int step_family_fused_n(niwqg_handle* h) {
         sa.y1q = h->y1q; sa.y1p = h->y1p; sa.F0q = h->F0q; sa.F0p = h->F0p; sa.Fabq = h->Fabq; sa.Fabp = h->Fabp;
         if (st == 1) { sa.yq = h->y1q; sa.yp = h->y1p; }     // the stage-1 state is written once, as y1 (read again at stage 3)
         sa.ph = h->ph; sa.tq = h->tq; sa.tp = h->tp; sa.filtr = h->filtr; sa.sumsD = h->sumsD; sa.partials = h->part;
-        fa.twc = h->twc; fa.dk = h->dk; fa.pf_next = h->fused_pf;
-        sa.hsym = (h->hsym && (h->p.use_filter || !h->p.dealias)) ? 1 : 0;
+        fa.twc = h->twc; fa.dk = h->dk;
+        sa.hsym = (h->p.use_filter || !h->p.dealias) ? 1 : 0;
         fa.T = h->T[0];
         { PROF(PK_SPEC); CK((launch_fstage<N>(fa, false, grid, h->stream))); }
         fa.T = h->T[1];
@@ -855,14 +829,7 @@ static int step_family_fused_n(niwqg_handle* h) {
             if ((r = split_rows(h, h->phix, h->phix, PRO_NONE, EPI_NONE, sc, true))) return r;
             if ((r = split_colsub(h, h->T[0], h->phiy, false))) return r;
             if ((r = split_rows(h, h->phiy, h->phiy, PRO_NONE, EPI_NONE, sc, true))) return r;
-            if (h->row_loader & 1) {
-                if ((r = split_rows_loader(h, LD_WAVEPV, h->W))) return r;
-            } else {
-                { PROF(PK_PHYS); k_phys_wavepv<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(h->phi, h->phix, h->phiy, h->W, h->npts, h->jscale); }
-                CK(cudaGetLastError());
-                h->launches++;
-                if ((r = split_rows(h, h->W, h->W, PRO_NONE, EPI_NONE, 1.0, false))) return r;
-            }
+            if ((r = split_rows_loader(h, LD_WAVEPV, h->W))) return r;
             if ((r = split_colsub(h, h->W, h->T[0], true))) return r;
         }
         // _invert(); _calc_rel_vorticity(); u, v
@@ -871,7 +838,7 @@ static int step_family_fused_n(niwqg_handle* h) {
         ia.i.filtr_sym = (h->p.use_filter || !h->p.dealias) ? 1 : 0;
         ia.i.ph = h->ph; ia.i.qs = h->qs; ia.i.W = h->T[0]; ia.i.qwh = (wave && st == 4) ? h->qwh : nullptr;
         ia.i.inv_jscale = 1.0 / h->jscale; ia.i.partials = h->part;
-        ia.T = h->T[0]; ia.out_uv = h->T[1]; ia.out_qs = h->T[2]; ia.twc = h->twc; ia.dk = h->dk; ia.pf_next = h->fused_pf;
+        ia.T = h->T[0]; ia.out_uv = h->T[1]; ia.out_qs = h->T[2]; ia.twc = h->twc; ia.dk = h->dk;
         { PROF(PK_SPEC); CK((launch_finvert<N>(ia, wave, grid, h->stream))); }
         h->launches++;
         FIN(SI_COUNT, h->sumsI, 0, grid);
@@ -893,8 +860,7 @@ static int step_family_fused(niwqg_handle* h) {
 }
 
 static int step_family(niwqg_handle* h) {
-    if (h->split && h->fused && (h->flags & MF_SPEC_BUDGET) && !(h->flags & (MF_YBJ | MF_QL_ADV)))
-        return step_family_fused(h);
+    if (h->split && (h->flags & MF_SPEC_BUDGET)) return step_family_fused(h);   // Coupled / UnCoupled
     const bool ybj = (h->flags & MF_YBJ) != 0, ql = (h->flags & MF_QL_ADV) != 0;
     const int oq = h->cq, op = h->cp;          // y0 buffers
     const int nq = ybj ? oq : 1 - oq, np = 1 - op;
@@ -908,7 +874,7 @@ static int step_family(niwqg_handle* h) {
         StageArgs sa{};
         sa.g = h->g;
         sa.stage = st; sa.flags = h->flags; sa.do_q = ybj ? 0 : 1; sa.do_phi = 1;
-        sa.hsym = (h->hsym && (h->p.use_filter || !h->p.dealias)) ? 1 : 0;
+        sa.hsym = (h->p.use_filter || !h->p.dealias) ? 1 : 0;
         sa.P1 = h->P1; sa.P2 = h->P2;
         sa.y0q = h->qh[oq]; sa.y0p = h->phih[op]; sa.yq = h->qh[nq]; sa.yp = h->phih[np];
         sa.y1q = h->y1q; sa.y1p = h->y1p; sa.F0q = h->F0q; sa.F0p = h->F0p; sa.Fabq = h->Fabq; sa.Fabp = h->Fabp;
@@ -930,17 +896,13 @@ static int step_family(niwqg_handle* h) {
                 sa.sums_here = 0;
                 { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream))); }
                 h->launches++;
-            } else if (h->split_stage) {
+            } else {
                 // two lighter kernels: q equation, then phi equation + the stage's spectral budget sums
                 sa.do_q = 1; sa.do_phi = 0; sa.sums_here = 0;
                 { PROF(PK_SPEC); CK((launch_spec_stage<true, false>(sa, pw_grid(h), h->stream))); }
                 sa.do_q = 0; sa.do_phi = 1; sa.sums_here = 1;
                 { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream))); }
                 h->launches += 2;
-            } else {
-                sa.sums_here = 1;
-                { PROF(PK_SPEC); CK((launch_spec_stage<true, true>(sa, pw_grid(h), h->stream))); }
-                h->launches++;
             }
             if (st == 1) { h->cq = nq; h->cp = np; }
         } else {
@@ -1221,12 +1183,6 @@ static int create_impl(niwqg_handle* h) {
     const niwqg_params& p = h->p;
     const int N = p.nx;
     CK(cudaSetDevice(p.device));
-    if (const char* e = getenv("NIWQG_PF_CTAS")) h->pf_ctas = atoi(e);   // tuning knob (0 = no prefetch)
-    if (const char* e = getenv("NIWQG_FFT_VARIANT")) h->fft_variant = atoi(e);
-    if (const char* e = getenv("NIWQG_TMA")) h->tma = atoi(e);
-    if (const char* e = getenv("NIWQG_SPLIT_STAGE")) h->split_stage = atoi(e);
-    if (const char* e = getenv("NIWQG_COL3")) h->col3 = atoi(e);
-    if (const char* e = getenv("NIWQG_HSYM")) h->hsym = atoi(e);
     CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&h->ev0));
     CK(cudaEventCreate(&h->ev1));
@@ -1245,19 +1201,14 @@ static int create_impl(niwqg_handle* h) {
     h->nk = h->qg ? N / 2 + 1 : h->ncl;
     h->npts = (size_t)h->nyl * N; h->nspec = (size_t)N * h->nk;
     h->Mg = (double)N * (double)N;
-    // de-interleaved physical x order (row pass = push kernel with contiguous stores): correct, but measured slower
-    // than the pull kernel on the natural layout (0.578 vs 0.535 ms per 8192^2 row pass), so it is opt-in
-    if (N > NIWQG_ROW_MAXM && getenv("NIWQG_DEINT")) { h->deintM = NIWQG_ROW_MAXM; h->deintC = N / NIWQG_ROW_MAXM; }
+    // the physical x order is de-interleaved on the split path only: for the cluster row pass (a push kernel with
+    // contiguous stores on that layout) it measured slower than the natural layout (0.578 vs 0.535 ms per 8192^2 row pass)
     if (h->nranks == 1 && h->B == 1 && !h->qg && N >= 2048) {
         const char* e = getenv("NIWQG_SPLIT");
         h->split = e ? (atoi(e) != 0) : (N == 8192);
-        if (const char* f = getenv("NIWQG_FUSED")) h->fused = atoi(f);
-        if (const char* f = getenv("NIWQG_ROW_BULK")) h->row_bulk = atoi(f);
-        if (const char* f = getenv("NIWQG_FUSED_PF")) h->fused_pf = atoi(f);
-        if (const char* f = getenv("NIWQG_ROW_LOADER")) h->row_loader = atoi(f);
-        if (const char* f = getenv("NIWQG_FUSED_GRID")) h->fused_grid = atoi(f);
         if (h->split) { h->deintM = N / 2; h->deintC = 2; }
     }
+    h->col3 = h->nranks == 1 && N == 8192 && h->B == 1 && !h->split;
     h->g = Grid{N, 2.0 * M_PI / p.L, h->ncl, h->ncl / 2, h->rank, h->nranks > 1 ? 1 : 0};
     if (h->nranks > 1) {
         int r = nccl_load(h->err);
@@ -1284,7 +1235,6 @@ static int create_impl(niwqg_handle* h) {
         default: h->flags = 0;
     }
     if (!h->qg && p.nu4w != 0.0) h->flags |= MF_HAS_LAP2;
-    if (getenv("NIWQG_NO_SPEC_BUDGET")) h->flags &= ~MF_SPEC_BUDGET;   // A/B knob: physical-space budget sums
     const size_t B = h->B, cb = sizeof(cd);
     const size_t fsz = B * h->npts * cb, ssz = B * h->nspec * cb, tsz = h->nspec * cb;
     // twiddles
@@ -1345,12 +1295,9 @@ static int create_impl(niwqg_handle* h) {
     h->lane_stream[0] = h->stream;
     h->lane_comm[0] = h->comm;
     // measured: 7% at 512^2, nothing at 2048^2, slightly negative at 8192^2 (the step is a chain of dependent kernels,
-    // ~5 us each whatever launches them) -> small grids only
-    {
-        int maxn = 1024;      // larger grids: kernels of 0.4-2 ms, the launch gaps a graph removes are noise (A/B knob)
-        if (const char* e = getenv("NIWQG_GRAPH_MAXN")) maxn = atoi(e);
-        h->use_graphs = (h->nranks == 1) && N <= maxn && !getenv("NIWQG_NO_GRAPH");
-    }
+    // ~5 us each whatever launches them; larger grids: kernels of 0.4-2 ms, the launch gaps a graph removes are noise)
+    // -> small grids only
+    h->use_graphs = (h->nranks == 1) && N <= 1024;
     if (h->split) {
         for (int o = 0; o < 3; ++o) DA(h->T[o], fsz);
         std::vector<cd> tw;
@@ -1362,41 +1309,26 @@ static int create_impl(niwqg_handle* h) {
         DA(h->tw_m, tw.size() * cb);
         CK(cudaMemcpyAsync(h->tw_m, tw.data(), tw.size() * cb, cudaMemcpyHostToDevice, h->stream));
         CK(cudaStreamSynchronize(h->stream));
-        h->col3 = 0;
     }
-    if (h->nranks == 1 && h->col3 && N == 8192 && B == 1) {
+    if (h->col3) {
         DA(h->S3[0], fsz); DA(h->S3[1], fsz);
         std::vector<cd> tw3;
         build_twiddles(512, tw3);
         DA(h->tw_c3, tw3.size() * cb);
         CK(cudaMemcpyAsync(h->tw_c3, tw3.data(), tw3.size() * cb, cudaMemcpyHostToDevice, h->stream));
         CK(cudaStreamSynchronize(h->stream));
-    } else {
-        h->col3 = 0;
     }
-    if (h->nranks == 1 && !getenv("NIWQG_ONE_LANE")) {
-        CK(cudaStreamCreateWithFlags(&h->lane_stream[1], cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-        h->lanes = true;
-    }
+    CK(cudaStreamCreateWithFlags(&h->lane_stream[1], cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     if (h->nranks > 1) {
         DA(h->X, fsz); DA(h->Y, fsz);
-        const int nl = getenv("NIWQG_ONE_LANE") ? 1 : niwqg_handle::NLANE;
-        if (const char* e = getenv("NIWQG_GROUP_OCC_LIMIT")) h->group_occ_limit = atoi(e);
-        if (const char* e = getenv("NIWQG_SLAB_BARRIER")) h->flag_barrier = strcmp(e, "nccl") != 0;
         h->slab_panel = (N >= NIWQG_COL_M && h->nyl >= N / NIWQG_COL_M && h->ncl % 4 == 0) ? N / NIWQG_COL_M : 0;
-        if (const char* e = getenv("NIWQG_SLAB_PANEL")) if (!atoi(e)) h->slab_panel = 0;
         // (+4 KB behind the first receive buffer of a lane: the barrier flags, mapped by the peers with the buffer)
-        for (int l = 0; l < nl; ++l) { DA(h->Yp[l][0], fsz + 4096); DA(h->Yp[l][1], fsz); DA(h->bar[l], 64); DA(h->Xl[l], fsz); }
+        for (int l = 0; l < niwqg_handle::NLANE; ++l) { DA(h->Yp[l][0], fsz + 4096); DA(h->Yp[l][1], fsz); DA(h->bar[l], 64); DA(h->Xl[l], fsz); }
+        if (const char* e = getenv("NIWQG_SLAB_BARRIER")) h->flag_barrier = strcmp(e, "nccl") != 0;
         if (const char* e = getenv("NIWQG_SLAB_EXCHANGE")) h->exchange = (strcmp(e, "ce") == 0) ? 1 : 0;
-        if (nl > 1) {
-            CK(cudaStreamCreateWithFlags(&h->lane_stream[1], cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-            NK(g_nccl.CommSplit(h->comm, 0, h->rank, &h->lane_comm[1], nullptr));
-            h->lanes = true;
-        }
+        NK(g_nccl.CommSplit(h->comm, 0, h->rank, &h->lane_comm[1], nullptr));
     }
     if (p.model != NIWQG_MODEL_YBJ) { DA(h->qh[1], ssz); DA(h->y1q, ssz); DA(h->F0q, ssz); DA(h->Fabq, ssz); }
     if (!h->qg) {

@@ -70,6 +70,22 @@ def test_product_path_never_imports_the_oracle():
                 assert "niwqg_oracle" not in src, "%s references the oracle module" % f
 
 
+def test_library_reads_no_tuning_switches_from_the_environment():
+    """The CUDA library chooses its algorithms from the problem (model, grid, batch, ranks), not from environment switches:
+    it reads NIWQG_SPLIT (the tests select the cluster-kernel reference path with it) and NIWQG_NCCL_LIB (where NCCL is).
+    NIWQG_SLAB_EXCHANGE and NIWQG_SLAB_BARRIER (copy-engine exchange, all-reduce barrier of slab runs) stay until their
+    removal has been checked on several GPUs."""
+    names = set()
+    for dirpath, _, files in os.walk(os.path.join(ROOT, "niwqg_b200", "csrc")):
+        for f in files:
+            src = open(os.path.join(dirpath, f)).read()
+            for arg in re.findall(r"getenv\s*\(([^)]*)\)", src):
+                m = re.fullmatch(r'\s*"(\w+)"\s*', arg)
+                assert m, "%s: getenv of a name that is not a literal: %s" % (f, arg)
+                names.add(m.group(1))
+    assert names == {"NIWQG_SPLIT", "NIWQG_NCCL_LIB", "NIWQG_SLAB_EXCHANGE", "NIWQG_SLAB_BARRIER"}, names
+
+
 def test_initial_conditions_match_reference_golden():
     """niwqg_b200.InitialConditions (host numpy, vectorised) reproduces the reference generators bit for bit:
     LambDipole against the q0 the unmodified reference produced (tests/golden/make_golden.py), the plane-wave /

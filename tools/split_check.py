@@ -1,5 +1,6 @@
 """Development aid: the split transform path (NIWQG_SPLIT=1) against the cluster path (NIWQG_SPLIT=0) on the same model
-runs: all four kernel-family models, N = 2048 (and 4096 / 8192 with --big), a few steps, field-level comparison."""
+runs: all four kernel-family models, N = 2048 (or the sizes given as arguments: Coupled only above 2048), a few steps,
+field-level comparison."""
 import os, sys, logging
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
@@ -8,8 +9,7 @@ logging.disable(logging.CRITICAL)
 from niwqg_b200 import CoupledModel, UnCoupledModel, YBJModel, QLModel
 from cases import lamb_params, rel_l2
 
-sizes = [int(a) for a in sys.argv[1:] if a.isdigit()] or [2048]
-extra = [a for a in sys.argv[1:] if not a.isdigit()]
+sizes = [int(a) for a in sys.argv[1:]] or [2048]
 worst = 0.0
 for nx in sizes:
     for name, mod in (("coupled", CoupledModel), ("uncoupled", UnCoupledModel), ("ybj", YBJModel), ("ql", QLModel)):
@@ -18,9 +18,6 @@ for nx in sizes:
         res = {}
         for split in ("0", "1"):
             os.environ["NIWQG_SPLIT"] = split
-            for e in extra:
-                k, v = e.split("=")
-                os.environ[k] = v if split == "1" else "0"
             kw, U0, k0 = lamb_params(nx, True, 2, 3)
             kw["twrite"] = 10 ** 9
             m = mod.Model(**kw)
