@@ -70,6 +70,11 @@ enum niwqg_field {
     NIWQG_F_EXPCH, NIWQG_F_EXPCH_H, NIWQG_F_QHCOEF, NIWQG_F_F0, NIWQG_F_FAB, NIWQG_F_FC,
     NIWQG_F_EXPCHW, NIWQG_F_EXPCH_HW, NIWQG_F_QHWCOEF, NIWQG_F_F0W, NIWQG_F_FABW, NIWQG_F_FCW,
     NIWQG_F_EXPCHC, NIWQG_F_EXPCH_HC, NIWQG_F_QHCCOEF, NIWQG_F_F0C, NIWQG_F_FABC, NIWQG_F_FCC,
+    /* carried physical buffers as the device holds them (complex (N,N)); Q, QW, QPSI, U, V are views of UV and QS */
+    NIWQG_F_UV,         /* u + i v                          */
+    NIWQG_F_QS,         /* q + i qw (Coupled/QL), q + i (q - q_psi) otherwise */
+    NIWQG_F_LAP2PHI,    /* ifft(wv4 phih) (models with nu4w != 0) */
+    NIWQG_F_UVQ,        /* QL: uq + i vq of the vortex flow */
     NIWQG_F_COUNT
 };
 
@@ -161,6 +166,24 @@ size_t niwqg_field_bytes(const niwqg_handle* h, int field);
  * further request waits for the staging buffer it needs. */
 int niwqg_get_field_async(niwqg_handle* h, int field, int member, void* dst, size_t bytes);
 int niwqg_wait_transfers(niwqg_handle* h);
+
+/* Checkpoint / exact restart (DESIGN.md section 6b).  The state of a handle is every buffer a step reads before it
+ * writes it, plus the scalar carry.  Restoring all of it into a handle of the same model, grid, batch and parameters
+ * makes the following steps bit-for-bit those of the handle it was read from.
+ *
+ * niwqg_state_slots: writes the field ids that make up this handle's state to ids[0..] and returns their number
+ * (at most 16; negative if max is too small).  Reading them with niwqg_get_field changes nothing on the device.
+ * niwqg_set_field: the inverse of niwqg_get_field for a state slot, same layout and size (natural x order, the rank's
+ * rows / column slab in a slab run, the half spectrum for QG).  Writes into the buffers of the current ping-pong
+ * parity; setting QH / PHIH marks the model seeded like set_q / set_phi.
+ * niwqg_carry_count / niwqg_get_carry / niwqg_set_carry: the per-member scalars a step carries into the next one
+ * (budgets Ke, Pw, Kw, cvar ... and the ep_psi sums of the last inversion), niwqg_carry_count(h) doubles.  In a slab
+ * run they are grid-wide and equal on every rank. */
+int niwqg_state_slots(const niwqg_handle* h, int* ids, int max);
+int niwqg_set_field(niwqg_handle* h, int field, int member, const void* src, size_t bytes, int on_device);
+int niwqg_carry_count(const niwqg_handle* h);
+int niwqg_get_carry(niwqg_handle* h, double* out);
+int niwqg_set_carry(niwqg_handle* h, const double* in);
 
 /* the FFT backend seam (niwqg/Kernel.py:553-566, niwqg/QGModel.py:536-552): one N x N
  * transform with numpy conventions, host buffers. */

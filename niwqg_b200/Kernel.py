@@ -11,6 +11,7 @@ import numpy as np
 from numpy import pi
 
 from . import _native as nat
+from . import Checkpoint
 from .Diagnostics import add_diagnostic, increment_diagnostics, get_diagnostic, describe_diagnostics  # noqa: F401
 from .Saving import initialize_save_snapshots, save_setup, save_snapshots, save_diagnostics
 
@@ -81,6 +82,12 @@ class Kernel(object):
 
     _model_id = None     # set by subclasses
     _ke = None
+    # constructor keywords a checkpoint records: the ones that reach the arithmetic (a restore requires them unchanged)
+    # and the ones that set the cadence and output of a run (from_checkpoint takes them over unless overridden)
+    _checkpoint_params = ("L", "dt", "U", "f", "N", "m", "g", "nu4", "nu4w", "nu", "nuw", "mu", "muw", "use_filter",
+                          "dealias")
+    _checkpoint_run = ("twrite", "tmax", "cflmax", "tdiags", "tsave_snapshots", "save_to_disk", "overwrite", "path")
+    _checkpoint_attr = {"tsave_snapshots": "tsnaps"}
 
     # device-backed attributes (names of the reference's numpy arrays)
     q = _DeviceField("Q"); qh = _DeviceField("QH"); p = _DeviceField("P"); ph = _DeviceField("PH")
@@ -278,6 +285,30 @@ class Kernel(object):
     def set_phi(self, phi=None):
         """niwqg/Kernel.py:538-551 (does not re-invert, F5).  ``phi=None``: the array queued with ``stage_inputs``."""
         self._h.set_phi(phi)
+
+    # ------------------------------------------------------------ checkpoint
+    def save_checkpoint(self, path, dist=None):
+        """Write the model's complete state to the directory ``path`` (niwqg_b200/Checkpoint.py): every carried device
+        field, Ke/Pw/Kw and the other scalars a step carries, t, tc, the diagnostics and the status attributes.  Changes
+        nothing on the model.  ``path`` must be new, empty or a checkpoint: another directory is never replaced.  Slab
+        runs call it on every rank (``dist``: torch.distributed, default the global one; an error on any rank is raised
+        on every rank)."""
+        Checkpoint.save(self, path, dist)
+
+    def load_checkpoint(self, path, dist=None):
+        """Restore a checkpoint written by ``save_checkpoint`` from a model of the same class, nx, batch and arithmetic
+        parameters (ValueError names any difference; the model is left as it was).  The steps that follow are
+        bit-for-bit those of the saved run; on another layout (slab ranks, split transforms) they agree to rounding.
+        ``dist`` as for save_checkpoint."""
+        Checkpoint.load(self, path, dist)
+
+    @classmethod
+    def from_checkpoint(cls, path, **overrides):
+        """The model saved in ``path``, built from its saved keywords and restored.  ``overrides`` replace keywords,
+        e.g. tmax, tdiags, path, device (or rank/nranks/nccl_id through slab.make_model).  Overriding an arithmetic
+        parameter such as dt or a dissipation coefficient is allowed, with a warning: the run then no longer continues
+        the saved one exactly."""
+        return Checkpoint.from_checkpoint(cls, path, **overrides)
 
     # ---------------------------------------------------------------- status
     def _print_status(self):

@@ -6,6 +6,7 @@ import numpy as np
 from numpy import pi
 
 from . import _native as nat
+from . import Checkpoint
 from .Kernel import _DeviceField, _Scalar, _LazyGrid, _wv2i
 from .Diagnostics import add_diagnostic, increment_diagnostics
 from .Saving import initialize_save_snapshots, save_setup, save_snapshots, save_diagnostics
@@ -20,6 +21,10 @@ class Model(object):
     expch = _DeviceField("EXPCH"); expch_h = _DeviceField("EXPCH_H"); Qh = _DeviceField("QHCOEF")
     f0 = _DeviceField("F0"); fab = _DeviceField("FAB"); fc = _DeviceField("FC")
     Ke = _Scalar("KE")
+    _checkpoint_params = ("L", "dt", "U", "nu4", "nu", "mu", "beta", "passive_scalar", "nu4c", "nuc", "muc",
+                          "use_filter", "dealias")
+    _checkpoint_run = ("twrite", "tswrite", "tmax", "tdiags", "tsave_snapshots", "save_to_disk", "overwrite", "path")
+    _checkpoint_attr = {"tsave_snapshots": "tsnaps"}
 
     def __init__(self, nx=128, ny=None, L=5e5, dt=10000., twrite=1000, tswrite=10, tmax=250000., use_filter=True,
                  U=.0, nu4=5.e9, nu=0, mu=0, beta=0, passive_scalar=False, nu4c=5.e9, nuc=0, muc=0, dealias=False,
@@ -165,6 +170,19 @@ class Model(object):
         if np.iscomplexobj(c):
             raise TypeError("set_c needs a real array (numpy.fft.rfft2 rejects complex input)")
         self._h.set_c(c)
+
+    def save_checkpoint(self, path):
+        """See Kernel.save_checkpoint."""
+        Checkpoint.save(self, path)
+
+    def load_checkpoint(self, path):
+        """See Kernel.load_checkpoint."""
+        Checkpoint.load(self, path)
+
+    @classmethod
+    def from_checkpoint(cls, path, **overrides):
+        """See Kernel.from_checkpoint."""
+        return Checkpoint.from_checkpoint(cls, path, **overrides)
 
     def _invert(self):
         """niwqg/QGModel.py:497-505: ph = -wv2i*qh is maintained on the device; nothing to do."""

@@ -19,11 +19,11 @@ MODEL_QG, MODEL_COUPLED, MODEL_UNCOUPLED, MODEL_YBJ, MODEL_QL = range(5)
 # enum niwqg_field
 FIELDS = ["Q", "QH", "PH", "P", "PHI", "PHIH", "PHIX", "PHIY", "LAPPHI", "U", "V", "QW", "QPSI", "QWH", "C", "CH",
           "FILTR", "EXPCH", "EXPCH_H", "QHCOEF", "F0", "FAB", "FC", "EXPCHW", "EXPCH_HW", "QHWCOEF", "F0W", "FABW",
-          "FCW", "EXPCHC", "EXPCH_HC", "QHCCOEF", "F0C", "FABC", "FCC"]
+          "FCW", "EXPCHC", "EXPCH_HC", "QHCCOEF", "F0C", "FABC", "FCC", "UV", "QS", "LAP2PHI", "UVQ"]
 F = {n: i for i, n in enumerate(FIELDS)}
 REAL_FIELDS = {"Q", "P", "U", "V", "QW", "QPSI", "C", "FILTR"}
-PHYS_CPLX_FIELDS = {"PHI", "PHIX", "PHIY", "LAPPHI"}
-TABLE_FIELDS = set(FIELDS[F["FILTR"]:])
+PHYS_CPLX_FIELDS = {"PHI", "PHIX", "PHIY", "LAPPHI", "UV", "QS", "LAP2PHI", "UVQ"}
+TABLE_FIELDS = set(FIELDS[F["FILTR"]:F["FCC"] + 1])
 
 # enum niwqg_scalar
 SCALARS = ["KE", "PW", "KW", "GAMMA1", "GAMMA2", "XI1", "XI2", "PI", "KE_QG", "ENS", "KE_NIW", "CKE_NIW", "IKE_NIW",
@@ -40,7 +40,8 @@ EXPORTS = ["niwqg_create", "niwqg_destroy", "niwqg_last_error", "niwqg_set_q", "
            "niwqg_field_bytes", "niwqg_fft2", "niwqg_jacobian", "niwqg_sync", "niwqg_time_steps",
            "niwqg_launch_count", "niwqg_stream", "niwqg_profile", "niwqg_nccl_unique_id", "niwqg_ic",
            "niwqg_get_field_async", "niwqg_wait_transfers", "niwqg_stage_q", "niwqg_stage_phi",
-           "niwqg_ipc_export", "niwqg_ipc_import", "niwqg_ipc_disable"]
+           "niwqg_ipc_export", "niwqg_ipc_import", "niwqg_ipc_disable", "niwqg_state_slots", "niwqg_set_field",
+           "niwqg_carry_count", "niwqg_get_carry", "niwqg_set_carry"]
 
 
 class Params(C.Structure):
@@ -96,6 +97,11 @@ def load():
     lib.niwqg_ipc_export.argtypes = [vp, vp, C.c_size_t]
     lib.niwqg_ipc_import.argtypes = [vp, vp, C.c_size_t]
     lib.niwqg_ipc_disable.argtypes = [vp]
+    lib.niwqg_state_slots.argtypes = [vp, vp, ip]
+    lib.niwqg_set_field.argtypes = [vp, ip, ip, vp, C.c_size_t, ip]
+    lib.niwqg_carry_count.argtypes = [vp]
+    lib.niwqg_get_carry.argtypes = [vp, vp]
+    lib.niwqg_set_carry.argtypes = [vp, vp]
     _lib = lib
     return lib
 
@@ -348,6 +354,31 @@ class Handle(object):
         if len(outs) == 1:
             return outs[0]
         return np.stack(outs)
+
+    # -- checkpoint / exact restart ---------------------------------------
+    def state_slots(self):
+        """Names of the fields that make up this handle's state (niwqg_state_slots)."""
+        ids = np.zeros(16, np.int32)
+        n = self.lib.niwqg_state_slots(self.h, ids.ctypes.data, ids.size)
+        if n < 0:
+            raise RuntimeError("niwqg_state_slots: more than %d slots" % ids.size)
+        return [FIELDS[i] for i in ids[:n]]
+
+    def set_field(self, name, member, a):
+        """Write one member's state slot, in the layout field() returns it (niwqg_set_field)."""
+        a = np.ascontiguousarray(a, np.float64 if name in REAL_FIELDS else np.complex128)
+        self._ck(self.lib.niwqg_set_field(self.h, F[name], member, a.ctypes.data, a.nbytes, 0))
+
+    def carry(self):
+        out = np.zeros(self.lib.niwqg_carry_count(self.h))
+        self._ck(self.lib.niwqg_get_carry(self.h, out.ctypes.data))
+        return out
+
+    def set_carry(self, a):
+        a = np.ascontiguousarray(a, np.float64)
+        if a.size != self.lib.niwqg_carry_count(self.h):
+            raise ValueError("expected %d carry values, got %d" % (self.lib.niwqg_carry_count(self.h), a.size))
+        self._ck(self.lib.niwqg_set_carry(self.h, a.ctypes.data))
 
     def field_to_device(self, name, member, ptr, nbytes):
         self._ck(self.lib.niwqg_get_field(self.h, F[name], member, C.c_void_p(ptr), nbytes, 1))

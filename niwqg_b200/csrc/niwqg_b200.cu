@@ -1924,7 +1924,8 @@ size_t niwqg_field_bytes(const niwqg_handle* h, int field) {
     switch (field) {
         case NIWQG_F_Q: case NIWQG_F_P: case NIWQG_F_U: case NIWQG_F_V: case NIWQG_F_QW: case NIWQG_F_QPSI: case NIWQG_F_C:
             return r;
-        case NIWQG_F_PHI: case NIWQG_F_PHIX: case NIWQG_F_PHIY: case NIWQG_F_LAPPHI: return c;
+        case NIWQG_F_PHI: case NIWQG_F_PHIX: case NIWQG_F_PHIY: case NIWQG_F_LAPPHI:
+        case NIWQG_F_UV: case NIWQG_F_QS: case NIWQG_F_LAP2PHI: case NIWQG_F_UVQ: return c;
         case NIWQG_F_FILTR: return h->nspec * sizeof(double);
         default: return s;
     }
@@ -1980,6 +1981,10 @@ static int get_field_impl(niwqg_handle* h, int field, int member, void* dst, siz
             }
             src = h->lapphi ? h->lapphi + mo : nullptr;
             break;
+        case NIWQG_F_UV: src = h->uv + mo; break;
+        case NIWQG_F_QS: src = h->qs + mo; break;
+        case NIWQG_F_LAP2PHI: src = h->lap2phi ? h->lap2phi + mo : nullptr; break;
+        case NIWQG_F_UVQ: src = h->uvq ? h->uvq + mo : nullptr; break;
         case NIWQG_F_QWH: src = h->qwh ? h->qwh + so : nullptr; break;
         case NIWQG_F_CH: src = h->chh[h->cc] ? h->chh[h->cc] + so : nullptr; break;
         case NIWQG_F_FILTR: src = h->filtr; break;
@@ -2010,6 +2015,7 @@ static int get_field_impl(niwqg_handle* h, int field, int member, void* dst, siz
             r = download_phys<double>(h, (const double*)src, dst, h->npts, on_device, (double*)h->P2, async);
             break;
         case NIWQG_F_PHI: case NIWQG_F_PHIX: case NIWQG_F_PHIY: case NIWQG_F_LAPPHI:
+        case NIWQG_F_UV: case NIWQG_F_QS: case NIWQG_F_LAP2PHI: case NIWQG_F_UVQ:
             r = download_phys<cd>(h, (const cd*)src, dst, h->npts, on_device, h->P2, async);
             break;
         default:
@@ -2031,6 +2037,110 @@ int niwqg_wait_transfers(niwqg_handle* h) {
     CK(cudaSetDevice(h->p.device));
     CK(cudaStreamSynchronize(h->copy_stream));
     CK(cudaStreamSynchronize(h->copy_out));
+    return 0;
+}
+
+// ---- checkpoint / exact restart: the state is every buffer a step (or the attribute and diagnostics reads that follow
+// it) reads before writing it.  Not state: y1/F0/Fab and the sums other than sumsI (written within a stage before they
+// are read), P1/P2/W/T/rscratch (scratch), lapphi of the spectral-budget models (recomputed wherever it is read).
+static const int MAX_SLOTS = 16;
+static int state_slots(const niwqg_handle* h, int* ids) {
+    int n = 0;
+    ids[n++] = NIWQG_F_QH;
+    ids[n++] = NIWQG_F_PH;
+    ids[n++] = NIWQG_F_UV;      // YBJ: u, v of set_q; QG: the stage-4 velocity that Gamma_c reads
+    ids[n++] = NIWQG_F_QS;      // physical q is the user's array after set_q (QG, YBJ) until it is next inverted
+    if (h->qg) {
+        if (h->p.passive_scalar) { ids[n++] = NIWQG_F_CH; ids[n++] = NIWQG_F_C; }   // C: W.x, the user's array after set_c
+        return n;
+    }
+    ids[n++] = NIWQG_F_PHIH;
+    ids[n++] = NIWQG_F_PHI;     // YBJ: refreshed at the end of a step only
+    ids[n++] = NIWQG_F_PHIX;    // UnCoupled / YBJ: refreshed at status and diagnostics ticks only (F6)
+    ids[n++] = NIWQG_F_PHIY;
+    if (h->flags & MF_WAVE_PV) ids[n++] = NIWQG_F_QWH;
+    if (!(h->flags & MF_SPEC_BUDGET)) {      // k_phys_rhs reads them; YBJ refreshes them at diagnostics ticks only
+        ids[n++] = NIWQG_F_LAPPHI;
+        if (h->flags & MF_HAS_LAP2) ids[n++] = NIWQG_F_LAP2PHI;
+    }
+    if (h->flags & MF_QL_ADV) ids[n++] = NIWQG_F_UVQ;   // read by the diagnostics pass
+    return n;
+}
+
+int niwqg_state_slots(const niwqg_handle* h, int* ids, int max) {
+    int all[MAX_SLOTS];
+    const int n = state_slots(h, all);
+    if (max < n) return -1;
+    for (int i = 0; i < n; ++i) ids[i] = all[i];
+    return n;
+}
+
+int niwqg_set_field(niwqg_handle* h, int field, int member, const void* src, size_t bytes, int on_device) {
+    CK(cudaSetDevice(h->p.device));
+    if (member < 0 || member >= h->B) { h->err = "set_field: bad member"; return -1; }
+    int ids[MAX_SLOTS];
+    const int n = state_slots(h, ids);
+    bool slot = false;
+    for (int i = 0; i < n; ++i) slot = slot || ids[i] == field;
+    if (!slot) { h->err = "set_field: not a state slot of this model"; return -1; }
+    if (bytes != niwqg_field_bytes(h, field)) { h->err = "set_field: size mismatch"; return -1; }
+    const size_t mo = (size_t)member * h->npts, so = (size_t)member * h->nspec;
+    cd* spec = nullptr;
+    cd* phys = nullptr;
+    switch (field) {
+        case NIWQG_F_QH: spec = h->qh[h->cq]; break;
+        case NIWQG_F_PHIH: spec = h->phih[h->cp]; break;
+        case NIWQG_F_CH: spec = h->chh[h->cc]; break;
+        case NIWQG_F_PH: spec = h->ph; break;
+        case NIWQG_F_QWH: spec = h->qwh; break;
+        case NIWQG_F_PHI: phys = h->phi; break;
+        case NIWQG_F_PHIX: phys = h->phix; break;
+        case NIWQG_F_PHIY: phys = h->phiy; break;
+        case NIWQG_F_LAPPHI: phys = h->lapphi; break;
+        case NIWQG_F_LAP2PHI: phys = h->lap2phi; break;
+        case NIWQG_F_UV: phys = h->uv; break;
+        case NIWQG_F_QS: phys = h->qs; break;
+        case NIWQG_F_UVQ: phys = h->uvq; break;
+        case NIWQG_F_C: {
+            int r = upload_phys<double>(h, src, h->rscratch + mo, h->npts, on_device);
+            if (r) return r;
+            k_real_to_cplx<<<NIWQG_PW_BLOCKS, NIWQG_PW_THREADS, 0, h->stream>>>(h->rscratch + mo, h->W + mo, h->npts);
+            CK(cudaGetLastError());
+            h->launches++;
+        } break;
+    }
+    if (spec) {
+        CK(cudaMemcpyAsync(spec + so, src, bytes, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, h->stream));
+        CK(cudaStreamSynchronize(h->stream));       // the caller may reuse its buffer when we return
+    }
+    if (phys) {
+        int r = upload_phys<cd>(h, src, phys + mo, h->npts, on_device);
+        if (r) return r;
+    }
+    if (field == NIWQG_F_QH) h->q_set = true;
+    if (field == NIWQG_F_PHIH) h->phi_set = true;
+    return 0;
+}
+
+// carry layout: scal [B][NIWQG_S_COUNT], then sumsI [B][SI_COUNT] (k_budget reads the sums of the previous step's last
+// inversion at stage 1)
+int niwqg_carry_count(const niwqg_handle* h) { return h->B * (NIWQG_S_COUNT + SI_COUNT); }
+
+int niwqg_get_carry(niwqg_handle* h, double* out) {
+    CK(cudaSetDevice(h->p.device));
+    const size_t ns = (size_t)h->B * NIWQG_S_COUNT;
+    CK(cudaMemcpyAsync(out, h->scal, ns * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(out + ns, h->sumsI, (size_t)h->B * SI_COUNT * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int niwqg_set_carry(niwqg_handle* h, const double* in) {
+    CK(cudaSetDevice(h->p.device));
+    const size_t ns = (size_t)h->B * NIWQG_S_COUNT;
+    CK(cudaMemcpyAsync(h->scal, in, ns * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->sumsI, in + ns, (size_t)h->B * SI_COUNT * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
 
