@@ -195,7 +195,10 @@ def test_8192_step_conserves_and_budgets_close():
 def test_cluster_transforms_are_bitwise_repeatable(N):
     """The cluster kernels exchange through distributed shared memory behind barriers; a missing barrier would show up
     as run-to-run differences (compute-sanitizer's racecheck is not available on the GPU pool).  Same input, several
-    back-to-back transforms (so different CTA placements and timings), bit-identical outputs, forward and inverse."""
+    back-to-back transforms (so different CTA placements and timings), bit-identical outputs, forward and inverse.
+    niwqg_fft2 transforms one member, and one member at 8192^2 takes the split transforms (fft2_split), so N = 8192
+    here exercises the split path; the full-grid 8192^2 cluster column pass runs only for batch > 1 and is repeated
+    bit for bit in tests/test_gpu_ensemble.py::test_8192_ensemble_matches_single_runs_and_repeats."""
     from niwqg_b200 import _native as nat
     h = nat.Handle(model=nat.MODEL_YBJ, nx=N, batch=1, device=0, L=5e5, dt=1e4, f=1e-4, N=0.01, m=0.025, nu=20., nuw=50.)
     rng = np.random.RandomState(11)

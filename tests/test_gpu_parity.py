@@ -6,7 +6,7 @@ steps (fp64 throughout); budgets are compared relative to their own magnitude.""
 import numpy as np
 import pytest
 
-from cases import CASES, EXTRA, lamb_params, load_golden, rel_l2
+from cases import CASES, case_ics, case_params, diag_check, lamb_params, load_golden, rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -23,25 +23,14 @@ def _models():
 def build_cuda(name, **over):
     import logging
     logging.disable(logging.CRITICAL)
-    from oracle import niwqg_oracle as orc
-    model, nx, use_filter, tdiags, nsteps, icname = CASES[name]
-    qg = model in ("qg", "qgc")
-    kw, U0, k0 = lamb_params(nx, use_filter, tdiags, nsteps, qg=qg)
-    if model == "qgc":
-        kw.update(passive_scalar=True, nu4c=3.e9 * (128 / nx) ** 4, nuc=0)
-    kw.update(EXTRA.get(name, {}))
-    kw.update(over)
+    model, kw, U0, k0 = case_params(name, **over)
     m = _models()[model](**kw)
-    if icname == "lamb":
-        q = orc.lamb_dipole(m, U=U0, R=2 * np.pi / k0)
-    else:
-        # the random IC needs the reference FFT arithmetic to be bit-identical: take it from the golden file
-        q = load_golden(name)["q0"]
-    m.set_q(q)
-    if model == "qgc":
-        m.set_c(np.exp(1j * (k0 / 5 * m.x + k0 / 5 * m.y) + 0.).real)
-    if not qg:
-        m.set_phi((np.ones_like(q) + 1j) * (2 * U0) / np.sqrt(2))
+    ics = case_ics(name, m, U0, k0)
+    m.set_q(ics["q"])
+    if "c" in ics:
+        m.set_c(ics["c"])
+    if "phi" in ics:
+        m.set_phi(ics["phi"])
     return m
 
 
@@ -139,45 +128,6 @@ def test_step_parity_against_reference_golden(name):
         assert abs(m.cvar - g["cvar"]) <= TOL_SCALAR * abs(g["cvar"])
 
 
-# Every diagnostic is compared against the magnitude of the budget it belongs to: cross terms and
-# tendencies are differences of much larger numbers, so "relative to itself" is not meaningful for them.
-QG_ENERGY = ("Ke", "ke_qg", "ke_qg_q", "ke_qg_w", "ke_qg_qw")
-WAVE_ENERGY = ("Kw", "ke_niw", "cke_niw", "ike_niw", "Pw", "pe_niw")
-TENDENCIES = ("gamma_r", "gamma_a", "xi_r", "xi_a", "pi", "ep_phi", "ep_psi", "chi_phi")
-SCALAR_TEND = ("ep_c", "chi_c", "Gamma_c")
-TOL_DIAG = 1e-9
-
-
-def _diag_scale(dn, ref, g):
-    def mx(names):
-        return max([float(np.max(np.abs(g["diag_" + n]))) for n in names if "diag_" + n in g] + [0.0])
-    if dn in ("skew", "conc_niw"):
-        return 1.0                                   # normalised O(1) quantities
-    if dn in QG_ENERGY:
-        return mx(("ke_qg",))
-    if dn in WAVE_ENERGY:
-        # Pw is compared on its own scale once it has grown; early on it is rounding noise of Kw
-        return max(float(np.max(np.abs(ref))), 1e-6 * mx(("ke_niw",)))
-    if dn in TENDENCIES:
-        return mx(TENDENCIES)
-    return float(np.max(np.abs(ref)))
-
-
-def _diag_check(name, dn, got, ref, g):
-    ref = np.asarray(ref, float); got = np.asarray(got, float)
-    assert got.shape == ref.shape, (dn, got.shape, ref.shape)
-    ok = np.isfinite(ref)                            # conc_niw is 0/0 for a uniform wave at t=0 in the reference too
-    ref, got = ref[ok], got[ok]
-    if ref.size == 0:
-        return
-    scale = _diag_scale(dn, ref, g)
-    if scale == 0:
-        assert np.max(np.abs(got)) < 1e-20, dn
-        return
-    err = float(np.max(np.abs(got - ref)) / scale)
-    assert err <= TOL_DIAG, (dn, err, got[:3], ref[:3])
-
-
 @pytest.mark.parametrize("name", ["coupled_lamb64_filt", "coupled_lamb64_nofilt", "uncoupled_lamb64_filt", "ql_lamb64_filt",
                                   "ybj_lamb64_filt", "coupled_rand64_filt", "coupled_lamb128_nofilt_100",
                                   "qg_lamb64_filt", "qg_scalar64_nofilt", "coupled_lamb64_diss", "coupled_lamb64_dealias",
@@ -190,7 +140,7 @@ def test_diagnostics_series_match_reference(name):
         if not k.startswith("diag_"):
             continue
         dn = k[5:]
-        _diag_check(name, dn, m.diagnostics[dn]['value'], ref, g)
+        diag_check(dn, m.diagnostics[dn]['value'], ref, g)
 
 
 def test_ensemble_members_match_single_runs():

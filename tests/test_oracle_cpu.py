@@ -78,3 +78,27 @@ def test_reference_fft_known_answers():
     m.set_q(g["qi"]); m.set_phi(g["phii"])
     assert float(m.spec_var(m.qh)) == float(g["spec_var_q"])
     assert abs(m.spec_var(m.phih) - g["phii"].var()) / g["phii"].var() < 1e-15
+
+
+def test_plane_wave_formula_matches_qg_oracle():
+    """The exact single-mode solution the GPU plane-wave tests use (cases.plane_wave_factor: hyperviscous decay,
+    Doppler shift and Rossby phase of the linear operator) against QGOracle stepping the same wave at 64^2."""
+    from cases import plane_wave_coefficient, plane_wave_factor
+    N, L, dt, nsteps, A = 64, 5e5, 2000., 3, 1e-14
+    x = (np.arange(N) + 0.5) / N * L
+    for kx, ky in ((5, 29), (29, 3), (17, 17)):
+        wv2 = (2 * np.pi / L) ** 2 * (kx * kx + ky * ky)
+        nu4 = 1.0 / (wv2 ** 2 * nsteps * dt)
+        beta = 0.5 * wv2 / (2 * np.pi / L * kx) / (nsteps * dt)
+        o = orc.QGOracle(nx=N, L=L, dt=dt, use_filter=False, nu4=nu4, nu=0., mu=0., beta=beta, U=0.03)
+        o.set_q(A * np.sin(2 * np.pi / L * (kx * x[None, :] + ky * x[:, None])))
+        want0 = plane_wave_coefficient(kx, ky, N, L, A)
+        assert abs(o.qh[ky, kx] - want0) <= 1e-13 * abs(want0)
+        for _ in range(nsteps):
+            o.step()
+        f = plane_wave_factor(kx, ky, N, L, nsteps * dt, nu4=nu4, beta=beta, U=0.03)
+        assert abs(np.angle(f)) > 0.1 and abs(f) < 0.5                  # the wave has moved and decayed
+        assert abs(o.qh[ky, kx] - want0 * f) <= 1e-12 * abs(want0 * f)
+        rest = o.qh.copy()
+        rest[ky, kx] = 0
+        assert np.abs(rest).max() <= 1e-9 * abs(want0 * f)     # the aliased 2K harmonic of the Jacobian, O(A)
