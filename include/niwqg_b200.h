@@ -1,9 +1,10 @@
 /* niwqg_b200.h -- C ABI of the B200-native ETDRK4 hot path of niwqg.
  *
  * Plain pointers and sizes only; no torch / C++ types.  One handle = one model
- * instance (optionally an ensemble of `batch` independent members that share
- * parameters) on one device and one CUDA stream.  All calls are asynchronous on
- * that stream except the ones that return data to the host.
+ * instance (optionally an ensemble of `batch` independent members that share the
+ * grid, time step and filter, and either share the physical coefficients or take
+ * their own: niwqg_create_ensemble) on one device and one CUDA stream.  All calls
+ * are asynchronous on that stream except the ones that return data to the host.
  *
  * Each entry point names the reference interface it replaces (paths relative to
  * the reference tree, cesar-rocha/niwqg).
@@ -32,7 +33,7 @@ typedef struct niwqg_params {
     size_t struct_size; /* = sizeof(niwqg_params): a binding built against another layout is rejected, not over-read */
     int model;          /* NIWQG_MODEL_*                                        */
     int nx;             /* grid edge, power of two, 32..8192 (ny==nx, F9)        */
-    int batch;          /* ensemble members sharing these parameters (>=1)       */
+    int batch;          /* ensemble members (>=1)                                */
     int device;         /* CUDA device ordinal                                   */
     double L, dt, U, f, N, m;
     double nu, nu4, mu;         /* q-equation dissipation                        */
@@ -48,6 +49,17 @@ typedef struct niwqg_params {
     int rank, nranks;
     char nccl_id[128];          /* ncclUniqueId from niwqg_nccl_unique_id() on rank 0, shared by the caller */
 } niwqg_params;
+
+/* the coefficients of niwqg_params that one member of an ensemble may set for itself (a parameter sweep in one
+ * batch); the other fields of niwqg_params - grid, dt, filter, model, slab layout - are common to all members */
+typedef struct niwqg_member_params {
+    size_t struct_size; /* = sizeof(niwqg_member_params) */
+    double U, f, N, m;
+    double nu, nu4, mu;         /* q-equation dissipation                        */
+    double nuw, nu4w, muw;      /* phi-equation dissipation                      */
+    double beta;                /* QGModel only                                  */
+    double nu4c, nuc, muc;      /* QGModel passive scalar                        */
+} niwqg_member_params;
 
 typedef struct niwqg_handle niwqg_handle;
 
@@ -65,7 +77,8 @@ enum niwqg_field {
     NIWQG_F_QPSI,       /* q_psi  real                      */
     NIWQG_F_QWH,        /* qwh    complex                   */
     NIWQG_F_C, NIWQG_F_CH,                                   /* QG passive scalar */
-    /* tables (shared by all members; member argument ignored) */
+    /* tables: FILTR is shared by all members (member argument ignored); the ETDRK4 tables of an equation are
+     * per member when the members' coefficients of that equation differ (niwqg_create_ensemble), else shared */
     NIWQG_F_FILTR,      /* real                             */
     NIWQG_F_EXPCH, NIWQG_F_EXPCH_H, NIWQG_F_QHCOEF, NIWQG_F_F0, NIWQG_F_FAB, NIWQG_F_FC,
     NIWQG_F_EXPCHW, NIWQG_F_EXPCH_HW, NIWQG_F_QHWCOEF, NIWQG_F_F0W, NIWQG_F_FABW, NIWQG_F_FCW,
@@ -101,6 +114,11 @@ enum niwqg_scalar {
  * (niwqg/QGModel.py:65-139): grid, filter (:267-284) and ETDRK4 tables (:400-454)
  * are generated on the device. */
 int niwqg_create(const niwqg_params* p, niwqg_handle** out);
+/* An ensemble whose members take their own coefficients: members[b] (p->batch entries) replaces the coefficient
+ * fields of p for member b; p gives everything else.  An equation (q, phi, passive scalar c) whose coefficients are
+ * equal in every member keeps one shared table set, any other gets one set per member (DESIGN.md section 3.3).
+ * members == NULL: exactly niwqg_create. */
+int niwqg_create_ensemble(const niwqg_params* p, const niwqg_member_params* members, niwqg_handle** out);
 int niwqg_destroy(niwqg_handle* h);
 const char* niwqg_last_error(const niwqg_handle* h);   /* h may be NULL: last create error */
 

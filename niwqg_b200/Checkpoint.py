@@ -250,11 +250,19 @@ def _class_name(cls):
 
 
 def _keywords(model, names):
+    """The model's keywords as JSON values: a per-member keyword (an array) becomes a list."""
     out = {}
     for k in names:
         v = getattr(model, model._checkpoint_attr.get(k, k))
-        out[k] = v.item() if isinstance(v, np.generic) else v
+        out[k] = v.tolist() if isinstance(v, np.ndarray) else (v.item() if isinstance(v, np.generic) else v)
     return out
+
+
+def _same(a, b):
+    """Keyword values a == b; lists (per-member values) element by element, and never equal to a scalar."""
+    if isinstance(a, (list, np.ndarray)) or isinstance(b, (list, np.ndarray)):
+        return np.shape(a) == np.shape(b) and bool(np.all(np.asarray(a) == np.asarray(b)))
+    return a == b
 
 
 def _io(model, dist):
@@ -290,7 +298,7 @@ def load(model, path, dist=None, changed=()):
             diffs.append("%s=%r (model: %r)" % (k, meta[k], getattr(model, k)))
     mine = _keywords(model, model._checkpoint_params)
     for k, v in sorted(meta["params"].items()):
-        if k not in changed and mine.get(k) != v:
+        if k not in changed and not _same(mine.get(k), v):
             diffs.append("%s=%r (model: %r)" % (k, v, mine.get(k)))
     if diffs:
         raise ValueError("checkpoint %s does not match the model: %s" % (path, ", ".join(diffs)))
@@ -322,7 +330,7 @@ def from_checkpoint(cls, path, dist=None, **overrides):
     meta = read_meta(path)
     if meta["model"] != _class_name(cls):
         raise ValueError("checkpoint %s holds a %s, not a %s" % (path, meta["model"], _class_name(cls)))
-    changed = sorted(k for k, v in overrides.items() if k in meta["params"] and v != meta["params"][k])
+    changed = sorted(k for k, v in overrides.items() if k in meta["params"] and not _same(v, meta["params"][k]))
     if changed:
         warnings.warn("restarting %s with %s changed: the run does not continue the saved one exactly"
                       % (path, ", ".join("%s=%r (was %r)" % (k, overrides[k], meta["params"][k]) for k in changed)))

@@ -73,6 +73,9 @@ class Kernel(object):
 
     Parameters are those of niwqg/Kernel.py:70-98 (SI units), plus
         batch  : number of independent ensemble members stepped together (default 1)
+    With batch > 1, each of U, f, N, m, nu, nu4, mu, nuw, nu4w, muw may be a sequence of batch values, one per member
+    (a parameter sweep in one batch; kappa, kappa2 and hslash are then arrays too).  nx, L, dt, use_filter, dealias
+    and g are common to all members.
         device : CUDA device ordinal (default 0)
         rank, nranks, nccl_id : slab decomposition of ONE grid over nranks GPUs (one process per GPU;
                  see niwqg_b200/slab.py).  set_q/set_phi then take the whole-grid array (each rank keeps its
@@ -117,6 +120,10 @@ class Kernel(object):
                  dealias=False, save_to_disk=False, overwrite=True, tsave_snapshots=10, tdiags=10,
                  path='output/', use_mkl=False, nthreads=1, batch=1, device=0, rank=0, nranks=1,
                  nccl_id=None):
+        kw = nat.member_keywords(batch, dict(U=U, f=f, N=N, m=m, nu=nu, nu4=nu4, mu=mu, nuw=nuw, nu4w=nu4w, muw=muw),
+                                 dict(nx=nx, L=L, dt=dt, use_filter=use_filter, dealias=dealias, g=g))
+        U, f, N, m, nu, nu4, mu, nuw, nu4w, muw = (kw[k] for k in ("U", "f", "N", "m", "nu", "nu4", "mu", "nuw", "nu4w",
+                                                                   "muw"))
         self.nx = nx
         self.ny = nx                    # niwqg/Kernel.py:100-103: ny is ignored (F9)
         self.L = L

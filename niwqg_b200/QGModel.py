@@ -13,7 +13,9 @@ from .Saving import initialize_save_snapshots, save_setup, save_snapshots, save_
 
 
 class Model(object):
-    """Parameters: niwqg/QGModel.py:65-91, plus ``batch`` and ``device``."""
+    """Parameters: niwqg/QGModel.py:65-91, plus ``batch`` and ``device``.  With batch > 1, each of U, beta, nu, nu4,
+    mu, nu4c, nuc, muc may be a sequence of batch values, one per member; nx, L, dt, use_filter, dealias and
+    passive_scalar are common to all members."""
 
     q = _DeviceField("Q"); qh = _DeviceField("QH"); p = _DeviceField("P"); ph = _DeviceField("PH")
     u = _DeviceField("U"); v = _DeviceField("V")
@@ -30,6 +32,10 @@ class Model(object):
                  U=.0, nu4=5.e9, nu=0, mu=0, beta=0, passive_scalar=False, nu4c=5.e9, nuc=0, muc=0, dealias=False,
                  save_to_disk=False, overwrite=True, tsave_snapshots=10, tdiags=10, path='output/', use_mkl=False,
                  nthreads=1, batch=1, device=0):
+        kw = nat.member_keywords(batch, dict(U=U, beta=beta, nu=nu, nu4=nu4, mu=mu, nu4c=nu4c, nuc=nuc, muc=muc),
+                                 dict(nx=nx, L=L, dt=dt, use_filter=use_filter, dealias=dealias,
+                                      passive_scalar=passive_scalar))
+        U, beta, nu, nu4, mu, nu4c, nuc, muc = (kw[k] for k in ("U", "beta", "nu", "nu4", "mu", "nu4c", "nuc", "muc"))
         self.nx = nx
         self.ny = nx
         self.L = L

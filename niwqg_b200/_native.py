@@ -24,6 +24,12 @@ F = {n: i for i, n in enumerate(FIELDS)}
 REAL_FIELDS = {"Q", "P", "U", "V", "QW", "QPSI", "C", "FILTR"}
 PHYS_CPLX_FIELDS = {"PHI", "PHIX", "PHIY", "LAPPHI", "UV", "QS", "LAP2PHI", "UVQ"}
 TABLE_FIELDS = set(FIELDS[F["FILTR"]:F["FCC"] + 1])
+# the equation (q, phi, passive scalar c) each ETDRK4 table field belongs to, and the constructor keywords that set that
+# equation's tables: the library gives an equation one table set per member when these differ between members
+TABLE_EQ = dict([(n, "q") for n in FIELDS[F["EXPCH"]:F["FC"] + 1]] + [(n, "phi") for n in FIELDS[F["EXPCHW"]:F["FCW"] + 1]] +
+                [(n, "c") for n in FIELDS[F["EXPCHC"]:F["FCC"] + 1]])
+TABLE_KEYS = {"q": ("U", "nu4", "nu", "mu", "beta"), "phi": ("U", "f", "N", "m", "nu4w", "nuw", "muw"),
+              "c": ("nu4c", "nuc", "muc")}
 
 # enum niwqg_scalar
 SCALARS = ["KE", "PW", "KW", "GAMMA1", "GAMMA2", "XI1", "XI2", "PI", "KE_QG", "ENS", "KE_NIW", "CKE_NIW", "IKE_NIW",
@@ -41,7 +47,7 @@ EXPORTS = ["niwqg_create", "niwqg_destroy", "niwqg_last_error", "niwqg_set_q", "
            "niwqg_launch_count", "niwqg_stream", "niwqg_profile", "niwqg_nccl_unique_id", "niwqg_ic",
            "niwqg_get_field_async", "niwqg_wait_transfers", "niwqg_stage_q", "niwqg_stage_phi",
            "niwqg_ipc_export", "niwqg_ipc_import", "niwqg_ipc_disable", "niwqg_state_slots", "niwqg_set_field",
-           "niwqg_carry_count", "niwqg_get_carry", "niwqg_set_carry"]
+           "niwqg_carry_count", "niwqg_get_carry", "niwqg_set_carry", "niwqg_create_ensemble"]
 
 
 class Params(C.Structure):
@@ -53,6 +59,35 @@ class Params(C.Structure):
                 ("use_filter", C.c_int), ("dealias", C.c_int), ("passive_scalar", C.c_int),
                 ("nu4c", C.c_double), ("nuc", C.c_double), ("muc", C.c_double),
                 ("rank", C.c_int), ("nranks", C.c_int), ("nccl_id", C.c_ubyte * 128)]
+
+
+# the coefficients one ensemble member may set for itself (struct niwqg_member_params)
+MEMBER_KEYS = ("U", "f", "N", "m", "nu", "nu4", "mu", "nuw", "nu4w", "muw", "beta", "nu4c", "nuc", "muc")
+
+
+class MemberParams(C.Structure):
+    _fields_ = [("struct_size", C.c_size_t)] + [(k, C.c_double) for k in MEMBER_KEYS]
+
+
+def member_keywords(batch, per_member, shared):
+    """Validate the constructor keywords of a model with ``batch`` members.  ``per_member``: {name: value}, each a
+    scalar (all members share it; returned unchanged) or a sequence of ``batch`` values (returned as a float64 array).
+    ``shared``: {name: value} that every member has in common, so a sequence there is an error.  ValueError names the
+    keyword."""
+    for k, v in shared.items():
+        if np.ndim(v) != 0:
+            raise ValueError("%s is common to all members of an ensemble: give one value, not a sequence" % k)
+    out = {}
+    for k, v in per_member.items():
+        if np.ndim(v) == 0:
+            out[k] = v
+            continue
+        a = np.asarray(v, dtype=np.float64)
+        if a.ndim != 1 or a.size != batch:
+            raise ValueError("%s: expected one value or a sequence of batch=%d values, got shape %s"
+                             % (k, batch, np.shape(v)))
+        out[k] = a
+    return out
 
 
 _lib = None
@@ -68,6 +103,7 @@ def load():
     lib = C.CDLL(LIB_PATH)
     vp, ip, dp = C.c_void_p, C.c_int, C.POINTER(C.c_double)
     lib.niwqg_create.argtypes = [C.POINTER(Params), C.POINTER(vp)]
+    lib.niwqg_create_ensemble.argtypes = [C.POINTER(Params), C.POINTER(MemberParams), C.POINTER(vp)]
     lib.niwqg_destroy.argtypes = [vp]
     lib.niwqg_last_error.argtypes = [vp]
     lib.niwqg_last_error.restype = C.c_char_p
@@ -160,7 +196,8 @@ def slab_owner(N, nranks, kx):
 
 
 class Handle(object):
-    """Owns one niwqg_handle.  Every method raises RuntimeError on a non-zero return."""
+    """Owns one niwqg_handle.  Every method raises RuntimeError on a non-zero return.  A keyword of MEMBER_KEYS given
+    as an array of ``batch`` values gives every member its own value (niwqg_create_ensemble)."""
 
     def __init__(self, **kw):
         path = _nccl_library_path() if kw.get("nranks", 1) > 1 else None
@@ -169,17 +206,31 @@ class Handle(object):
         self.lib = load()
         p = Params()
         p.struct_size = C.sizeof(Params)
+        swept = {k: np.asarray(v, np.float64) for k, v in kw.items() if k in MEMBER_KEYS and np.ndim(v) != 0}
         for k, v in kw.items():
             if k == "nccl_id":      # raw 128 bytes (a c_char array would stop at the first NUL)
                 if v is None or len(v) != 128:
                     raise ValueError("nccl_id must be the 128 bytes of nccl_unique_id()")
                 C.memmove(C.addressof(p) + Params.nccl_id.offset, bytes(v), 128)
             else:
-                setattr(p, k, v)
+                setattr(p, k, float(swept[k][0]) if k in swept else v)
+        members = None
+        if swept:
+            for k, v in swept.items():
+                if v.shape != (p.batch,):
+                    raise ValueError("%s: expected %d per-member values, got shape %s" % (k, p.batch, v.shape))
+            members = (MemberParams * p.batch)()
+            for b in range(p.batch):
+                members[b].struct_size = C.sizeof(MemberParams)
+                for k in MEMBER_KEYS:
+                    setattr(members[b], k, float(swept[k][b]) if k in swept else getattr(p, k))
+        # equations whose tables the library holds per member (its rule: the equation's keywords differ)
+        eqs = ("q", "c") if p.model == MODEL_QG else ("q", "phi")
+        self.table_members = {eq for eq in eqs if any(k in swept and np.any(swept[k] != swept[k][0]) for k in TABLE_KEYS[eq])}
         self.params = p
         self._staged = {}
         self.h = C.c_void_p()
-        rc = self.lib.niwqg_create(C.byref(p), C.byref(self.h))
+        rc = self.lib.niwqg_create_ensemble(C.byref(p), members, C.byref(self.h))
         if rc != 0:
             msg = self.lib.niwqg_last_error(None)
             self.h = None
@@ -345,7 +396,11 @@ class Handle(object):
             shape, dt = (self.nyl, N), np.complex128
         else:
             shape, dt = (N, nk), np.complex128
-        members = [0] if (name in TABLE_FIELDS) else (range(self.B) if member is None else [member])
+        if name in TABLE_FIELDS:     # shared tables: one array; per-member tables: a member axis as for the state
+            pm = TABLE_EQ.get(name) in self.table_members
+            members = (range(self.B) if member is None else [member]) if pm else [0]
+        else:
+            members = range(self.B) if member is None else [member]
         outs = []
         for mm in members:
             a = np.empty(shape, dt)

@@ -74,6 +74,14 @@ __device__ void etdrk4_point(cd ch, double dt, cd& E, cd& E2, cd& Q, cd& f0, cd&
 
 struct TableSet { cd *E, *E2, *Q, *f0, *fab, *fc; };
 
+// Per-member coefficients the kernels read by value of blockIdx.y: mcoef[member][MC_COUNT] (equal rows when the
+// members share their parameters).  MC_PW_SEED = 0.25 / (N^2 kappa2), the Pw of set_phi per unit grad^2 sum.
+enum { MC_F = 0, MC_HSLASH, MC_KAPPA2, MC_NU4, MC_NU, MC_MU, MC_NU4W, MC_NUW, MC_MUW, MC_NU4C, MC_MUC, MC_PW_SEED,
+       MC_COUNT };
+
+// coefficients of one equation's exponent c (see InitArgs), per member for k_init_tables
+enum { IC_RE_A4 = 0, IC_RE_A2, IC_RE_A0, IC_IM_WV2, IC_BETA, IC_U, IC_COUNT };
+
 struct InitArgs {
     Grid g;                  // slab column map (kernel family); g.sym == 0 for the natural layout
     int N, nk;               // nk = local spectral columns: N (c2c), N/P (slab) or N/2+1 (QG half spectrum)
@@ -86,23 +94,33 @@ struct InitArgs {
     int use_filter, dealias;
     TableSet t;
     double* filtr;               // may be null
+    const double* mc;            // null: one table set from the scalars above; else [gridDim.y][IC_COUNT], one set per
+                                 // member (blockIdx.y) at offset member * N * nk of every table
 };
 
 __global__ void k_init_tables(InitArgs a) {
     const size_t total = (size_t)a.N * a.nk;
+    double re_a4 = a.re_a4, re_a2 = a.re_a2, re_a0 = a.re_a0, im_wv2 = a.im_wv2, beta = a.beta, U = a.U;
+    size_t mo = 0;
+    if (a.mc) {
+        const double* c = a.mc + (size_t)blockIdx.y * IC_COUNT;
+        re_a4 = c[IC_RE_A4]; re_a2 = c[IC_RE_A2]; re_a0 = c[IC_RE_A0]; im_wv2 = c[IC_IM_WV2]; beta = c[IC_BETA]; U = c[IC_U];
+        mo = (size_t)blockIdx.y * total;
+    }
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const int row = (int)(i / a.nk), col = (int)(i % a.nk);
         const double k = a.dk * (double)(a.half ? col : sidx(grid_kx(a.g, col), a.N));
         const double l = a.dk * (double)sidx(row, a.N);
         const double wv2 = __dadd_rn(__dmul_rn(k, k), __dmul_rn(l, l));
         const double wv4 = __dmul_rn(wv2, wv2);
-        double cre = __dsub_rn(__dsub_rn(__dmul_rn(-a.re_a4, wv4), __dmul_rn(a.re_a2, wv2)), a.re_a0);
-        double cim = __dsub_rn(-__dmul_rn(k, a.U), __dmul_rn(a.im_wv2, wv2));
-        if (a.beta != 0.0 && wv2 != 0.0) cim += a.beta * k * (1.0 / wv2);   // QGModel.py:428
+        double cre = __dsub_rn(__dsub_rn(__dmul_rn(-re_a4, wv4), __dmul_rn(re_a2, wv2)), re_a0);
+        double cim = __dsub_rn(-__dmul_rn(k, U), __dmul_rn(im_wv2, wv2));
+        if (beta != 0.0 && wv2 != 0.0) cim += beta * k * (1.0 / wv2);   // QGModel.py:428
         cd E, E2, Q, f0, fab, fc;
         etdrk4_point(make_double2(cre * a.dt, cim * a.dt), a.dt, E, E2, Q, f0, fab, fc);
-        a.t.E[i] = E; a.t.E2[i] = E2; a.t.Q[i] = Q; a.t.f0[i] = f0; a.t.fab[i] = fab; a.t.fc[i] = fc;
-        if (a.filtr) {
+        const size_t j = mo + i;
+        a.t.E[j] = E; a.t.E2[j] = E2; a.t.Q[j] = Q; a.t.f0[j] = f0; a.t.fab[j] = fab; a.t.fc[j] = fc;
+        if (a.filtr && blockIdx.y == 0) {
             double fl = 1.0;
             if (a.use_filter) {
                 const double cphi = 0.65 * 3.14159265358979323846;
@@ -177,10 +195,12 @@ __device__ __forceinline__ void pack_uv_general(double k1, double l1, double k2,
     out2 = make_double2(HU.x + HV.y, -HU.y + HV.x);
 }
 
-__global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_invert(InvertArgs a) {
+// mcoef: [member][MC_COUNT] (this kernel reads the member's f instead of a.f, which the batch-1 fused inversion uses)
+__global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_invert(InvertArgs a, const double* __restrict__ mcoef) {
     double s[SI_COUNT] = {0.0, 0.0, 0.0};
     const int N = a.g.N, H = N >> 1, NC = a.g.ncl;
     const size_t npts = (size_t)N * NC, mb = (size_t)blockIdx.y * npts;
+    const double f = mcoef[(size_t)blockIdx.y * MC_COUNT + MC_F];
     const size_t total = (size_t)(H + 1) * NC;
     for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
         const int ky = (int)(t / NC), lc = (int)(t % NC);
@@ -217,8 +237,8 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_invert(InvertArgs a) 
             fl1 = a.filtr[(size_t)ky * NC + lc];
             fl2 = a.filtr_sym ? fl1 : a.filtr[(size_t)kyp * NC + lcp];
             const double fs = 0.5 * (fl1 + fl2);
-            qwb.x = 0.5 * (0.5 * (-wv2 * A.x) + Jc.x) / a.f;
-            qwb.y = 0.5 * (0.5 * (-wv2 * A.y) + Jc.y) / a.f;
+            qwb.x = 0.5 * (0.5 * (-wv2 * A.x) + Jc.x) / f;
+            qwb.y = 0.5 * (0.5 * (-wv2 * A.y) + Jc.y) / f;
             qw.x = qwb.x * fs;
             qw.y = qwb.y * fs;
         }
@@ -293,7 +313,7 @@ enum {
 struct PhysArgs {
     size_t npts;
     int flags;
-    double nu4w, nuw, muw;
+    const double* mcoef;      // [member][MC_COUNT]: nu4w, nuw, muw of diss
     const cd *uv, *qs, *phi, *phix, *phiy, *lapphi, *lap2phi, *uvq;
     cd *P1, *P2;
     double* partials;
@@ -331,11 +351,14 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_phys_rhs(PhysArgs a) {
         s[SD_QP2] += qpsi * qpsi;
         s[SD_QP3] += qpsi * qpsi * qpsi;
         if (a.flags & MF_SPEC_BUDGET) continue;      // the lapphi terms come from k_spec_stage
+        const double* mc = a.mcoef + (size_t)blockIdx.y * MC_COUNT;
+        const double nuw = mc[MC_NUW], muw = mc[MC_MUW];
         const cd lp = a.lapphi[mb + i];
-        cd diss = make_double2(a.nuw * lp.x - a.muw * phi.x, a.nuw * lp.y - a.muw * phi.y);
+        cd diss = make_double2(nuw * lp.x - muw * phi.x, nuw * lp.y - muw * phi.y);
         if (a.flags & MF_HAS_LAP2) {
+            const double nu4w = mc[MC_NU4W];
             const cd l2 = a.lap2phi[mb + i];
-            diss.x += -a.nu4w * l2.x; diss.y += -a.nu4w * l2.y;
+            diss.x += -nu4w * l2.x; diss.y += -nu4w * l2.y;
         }
         s[SD_G1] += qpsi * (phi.x * lp.y - phi.y * lp.x);            // Im(conj(phi) lap)
         s[SD_G2] += lp.x * J.x + lp.y * J.y;                          // Re(conj(lap) J)
@@ -415,8 +438,9 @@ __device__ __forceinline__ cd etd_update(int stage, cd y0, cd y1, cd Fn, cd& F0,
 // ST (stage 1..4), DQ / DP (update the q / phi equation) are compile-time so that every instantiation carries only
 // the loads of its stage and equation.  Every launch updates one equation: a body that updated both needed 128 registers
 // and ran at ~79 % of the HBM peak, the two halves launched back to back are lighter and faster (they share only the 8 B
-// filter value).
-template <int ST, bool DQ, bool DP>
+// filter value).  PM: the updated equation's tables hold one set per member (a parameter sweep), indexed like the state;
+// otherwise one shared set indexed by the wavenumber alone.
+template <int ST, bool DQ, bool DP, bool PM>
 __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
     const int N = a.g.N, H = N >> 1, NC = a.g.ncl;
     const size_t npts = (size_t)N * NC, mb = (size_t)blockIdx.y * npts;
@@ -467,12 +491,12 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
             if (st >= 3) { Faba = a.Fabp[i1]; Fabb = a.Fabp[i2]; }
             if (st == 3) { y1a = a.y1p[i1]; y1b = a.y1p[i2]; }
             const cd b1 = (st == 1) ? cur1 : a.y0p[i1], b2 = (st == 1) ? cur2 : a.y0p[i2];
-            const cd n1 = etd_update(st, b1, y1a, F1, F0a, Faba, a.tp, t1, fl1);
+            const cd n1 = etd_update(st, b1, y1a, F1, F0a, Faba, a.tp, PM ? i1 : t1, fl1);
             a.yp[i1] = n1;
             if (st == 1) { a.F0p[i1] = F0a; a.y1p[i1] = n1; }
             if (st == 2 || st == 3) a.Fabp[i1] = Faba;
             if (!self) {
-                const cd n2 = etd_update(st, b2, y1b, F2, F0b, Fabb, a.tp, t2, fl2);
+                const cd n2 = etd_update(st, b2, y1b, F2, F0b, Fabb, a.tp, PM ? i2 : t2, fl2);
                 a.yp[i2] = n2;
                 if (st == 1) { a.F0p[i2] = F0b; a.y1p[i2] = n2; }
                 if (st == 2 || st == 3) a.Fabp[i2] = Fabb;
@@ -501,7 +525,7 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
             if (st == 3) { y1a = a.y1q[i1]; if (!hs) y1b = a.y1q[i2]; }
             const cd b1 = a.y0q[i1];                       // the ep_psi sums of this state: k_spec_invert
             if (!hs) b2 = a.y0q[i2];
-            const cd n1 = etd_update(st, b1, y1a, F1, F0a, Faba, a.tq, t1, fl1);
+            const cd n1 = etd_update(st, b1, y1a, F1, F0a, Faba, a.tq, PM ? i1 : t1, fl1);
             a.yq[i1] = n1;
             if (st == 1) { a.F0q[i1] = F0a; a.y1q[i1] = n1; }
             if (st == 2 || st == 3) a.Fabq[i1] = Faba;
@@ -511,7 +535,7 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
                     n2 = make_double2(n1.x, -n1.y);
                     F0b = make_double2(F0a.x, -F0a.y);
                     Fabb = make_double2(Faba.x, -Faba.y);
-                } else n2 = etd_update(st, b2, y1b, F2, F0b, Fabb, a.tq, t2, fl2);
+                } else n2 = etd_update(st, b2, y1b, F2, F0b, Fabb, a.tq, PM ? i2 : t2, fl2);
                 a.yq[i2] = n2;
                 if (st == 1) { a.F0q[i2] = F0b; a.y1q[i2] = n2; }
                 if (st == 2 || st == 3) a.Fabq[i2] = Fabb;
@@ -521,14 +545,20 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_spec_stage(StageArgs a) {
     if (a.sums_here) block_reduce_store<SE_COUNT>(s, a.partials);
 }
 
-template <bool DQ, bool DP>
-static cudaError_t launch_spec_stage(const StageArgs& a, dim3 grid, cudaStream_t st) {
+template <bool DQ, bool DP, bool PM>
+static void launch_spec_stage_pm(const StageArgs& a, dim3 grid, cudaStream_t st) {
     switch (a.stage) {
-        case 1: k_spec_stage<1, DQ, DP><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
-        case 2: k_spec_stage<2, DQ, DP><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
-        case 3: k_spec_stage<3, DQ, DP><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
-        default: k_spec_stage<4, DQ, DP><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
+        case 1: k_spec_stage<1, DQ, DP, PM><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
+        case 2: k_spec_stage<2, DQ, DP, PM><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
+        case 3: k_spec_stage<3, DQ, DP, PM><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
+        default: k_spec_stage<4, DQ, DP, PM><<<grid, NIWQG_PW_THREADS, 0, st>>>(a); break;
     }
+}
+// pm: the tables of the equation this launch updates are per member
+template <bool DQ, bool DP>
+static cudaError_t launch_spec_stage(const StageArgs& a, dim3 grid, cudaStream_t st, bool pm) {
+    if (pm) launch_spec_stage_pm<DQ, DP, true>(a, grid, st);
+    else launch_spec_stage_pm<DQ, DP, false>(a, grid, st);
     return cudaGetLastError();
 }
 
@@ -539,8 +569,8 @@ static cudaError_t launch_spec_stage(const StageArgs& a, dim3 grid, cudaStream_t
 struct BudgetArgs {
     int stage;           // 1..4 ; 0 = evaluate only (diagnostics tick)
     double M;            // N*N
-    double f, hslash, kappa2, dt;
-    double nu4, nu, mu, nu4w, nuw, muw;
+    double dt;
+    const double* mcoef; // [member][MC_COUNT]: f, hslash, kappa2 and the dissipation coefficients
     const double *sumsD, *sumsE, *sumsI;   // physical (k_phys_rhs), stage-spectral (k_spec_stage), k_spec_invert
     int spec_budget;
     double* scal;        // [member][NIWQG_S_COUNT]

@@ -164,6 +164,8 @@ __device__ __forceinline__ cd qg_update_point(int st, const cd* y0, cd* y, cd* y
     return n;
 }
 
+// PMQ / PMC: the q / c tables hold one set per member (a parameter sweep), indexed like the state
+template <bool PMQ, bool PMC>
 __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_qg_stage(QgStageArgs a) {
     const int N = a.N, nk = a.nk, H = N >> 1, st = a.stage;
     const size_t npts = (size_t)N * N, nspec = (size_t)N * nk;
@@ -182,11 +184,11 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_qg_stage(QgStageArgs a) {
         const double wv2 = k * k + l1 * l1;      // same for both members of an edge pair
         const double wv2i = (wv2 != 0.0) ? 1.0 / wv2 : 0.0;
         // ---- q equation
-        const cd qn1 = qg_update_point(st, a.y0q, a.yq, a.y1q, a.F0q, a.Fabq, a.tq, mbh + t1, t1,
+        const cd qn1 = qg_update_point(st, a.y0q, a.yq, a.y1q, a.F0q, a.Fabq, a.tq, mbh + t1, PMQ ? mbh + t1 : t1,
                                        qg_neg_jac(a.P1, mbf, N, ky, kx, k, l1), a.filtr[t1]);
         cd qn2 = qn1;
         if (pair)
-            qn2 = qg_update_point(st, a.y0q, a.yq, a.y1q, a.F0q, a.Fabq, a.tq, mbh + t2, t2,
+            qn2 = qg_update_point(st, a.y0q, a.yq, a.y1q, a.F0q, a.Fabq, a.tq, mbh + t2, PMQ ? mbh + t2 : t2,
                                   qg_neg_jac(a.P1, mbf, N, kyp, kx, k, l2), a.filtr[t2]);
         // ---- ep_psi on (new qh, new ph, stale q):  stale q is y0 for stages 1-3, the new qh for stage 4
         {
@@ -208,11 +210,11 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_qg_stage(QgStageArgs a) {
         }
         if (!a.ps) continue;
         // ---- passive scalar
-        const cd cn1 = qg_update_point(st, a.y0c, a.yc, a.y1c, a.F0c, a.Fabc, a.tc, mbh + t1, t1,
+        const cd cn1 = qg_update_point(st, a.y0c, a.yc, a.y1c, a.F0c, a.Fabc, a.tc, mbh + t1, PMC ? mbh + t1 : t1,
                                        qg_neg_jac(a.P2, mbf, N, ky, kx, k, l1), a.filtr[t1]);
         cd cn2 = cn1;
         if (pair)
-            cn2 = qg_update_point(st, a.y0c, a.yc, a.y1c, a.F0c, a.Fabc, a.tc, mbh + t2, t2,
+            cn2 = qg_update_point(st, a.y0c, a.yc, a.y1c, a.F0c, a.Fabc, a.tc, mbh + t2, PMC ? mbh + t2 : t2,
                                   qg_neg_jac(a.P2, mbf, N, kyp, kx, k, l2), a.filtr[t2]);
         {
             // C2 = spec_var(ch), gradC2 = spec_var(wv ch): weights 2 (interior) / 1 (edge columns), no projection (QGModel.py:611-619)
@@ -233,7 +235,8 @@ __global__ void __launch_bounds__(NIWQG_PW_THREADS) k_qg_stage(QgStageArgs a) {
 
 struct QgBudgetArgs {
     int stage, ps;
-    double M, dt, nu4, nu, mu, nu4c, muc;
+    double M, dt;
+    const double* mcoef;     // [member][MC_COUNT]: nu4, nu, mu, nu4c, muc
     const double* sumsE;
     double *scal, *stagev;
 };
@@ -242,12 +245,14 @@ __global__ void k_qg_budget(QgBudgetArgs a) {
     const int m = blockIdx.x;
     if (threadIdx.x != 0) return;
     const double* se = a.sumsE + (size_t)m * QE_COUNT;
+    const double* mc = a.mcoef + (size_t)m * MC_COUNT;
     double* sc = a.scal + (size_t)m * NIWQG_S_COUNT;
     double* sv = a.stagev + (size_t)m * 12 + (a.stage - 1) * 3;
     const double M2 = a.M * a.M;
-    sv[0] = a.nu4 * (se[QE_QLAP2PSI] / M2) - a.nu * (se[QE_PLAPQ] / M2) + a.mu * (se[QE_PQ] / M2);   // QGModel.py:588-593
+    const double nu4 = mc[MC_NU4], nu = mc[MC_NU], mu = mc[MC_MU], nu4c = mc[MC_NU4C], muc = mc[MC_MUC];
+    sv[0] = nu4 * (se[QE_QLAP2PSI] / M2) - nu * (se[QE_PLAPQ] / M2) + mu * (se[QE_PQ] / M2);   // QGModel.py:588-593
     // ep_c uses self.nu for the gradient term (QGModel.py:597)
-    sv[1] = a.ps ? (-2 * a.nu4c * (se[QE_LAPC2] / M2) - 2 * a.nu * (se[QE_GRADC2] / M2) - 2 * a.muc * (se[QE_C2] / M2)) : 0.0;
+    sv[1] = a.ps ? (-2 * nu4c * (se[QE_LAPC2] / M2) - 2 * nu * (se[QE_GRADC2] / M2) - 2 * muc * (se[QE_C2] / M2)) : 0.0;
     if (a.stage == 4) {
         const double* s0 = a.stagev + (size_t)m * 12;
         sc[NIWQG_S_KE] += a.dt * (s0[0] + 2 * (s0[3] + s0[6]) + s0[9]) / 6.;

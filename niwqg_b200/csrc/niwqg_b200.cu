@@ -39,7 +39,13 @@ struct niwqg_handle {
     bool qg = false;
     int nk = 0;                 // spectral row length: N (c2c) or N/2+1 (QG)
     size_t npts = 0, nspec = 0; // N*N, N*nk
-    double dk = 0, dx = 0, kappa2 = 0, hslash = 0, jscale = 1.0;
+    double dk = 0, dx = 0, jscale = 1.0;
+    // per-member coefficients (niwqg_create_ensemble; copies of p otherwise): host rows for the finalisation of
+    // diagnostics / status, device rows mcoef[B][MC_COUNT] for the kernels
+    std::vector<niwqg_member_params> mp;
+    std::vector<double> kappa2m, hslashm;
+    double* mcoef = nullptr;
+    bool pm_q = false, pm_p = false, pm_c = false;   // per-member tables of the q / phi / c equation
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::vector<void*> allocs;
@@ -605,28 +611,31 @@ __global__ void k_budget(BudgetArgs a) {
     const double* sd = a.sumsD + (size_t)m * SD_COUNT;
     const double* se = a.sumsE + (size_t)m * SE_COUNT;
     const double* si = a.sumsI + (size_t)m * SI_COUNT;
+    const double* mc = a.mcoef + (size_t)m * MC_COUNT;
     double* sc = a.scal + (size_t)m * NIWQG_S_COUNT;
     const double M = a.M, M2 = M * M;
+    const double f = mc[MC_F], hslash = mc[MC_HSLASH], kappa2 = mc[MC_KAPPA2];
+    const double nu4 = mc[MC_NU4], nu = mc[MC_NU], mu = mc[MC_MU], nu4w = mc[MC_NU4W], nuw = mc[MC_NUW], muw = mc[MC_MUW];
     double g1, g2, x1, x2, lap2m;
     if (a.spec_budget) {
         // only the sums gamma1+gamma2 and xi1+xi2 enter the stage tendencies (Kernel.py:320-321); Parseval forms
-        g1 = 0.5 * a.hslash * (se[SE_T1R] / M2) / a.f;
+        g1 = 0.5 * hslash * (se[SE_T1R] / M2) / f;
         g2 = 0.0;
-        x1 = ((-a.nu4w * se[SE_T2I] - a.nuw * se[SE_T1I] - a.muw * se[SE_T0I]) / M2) / a.f;
+        x1 = ((-nu4w * se[SE_T2I] - nuw * se[SE_T1I] - muw * se[SE_T0I]) / M2) / f;
         x2 = 0.0;
         lap2m = se[SE_LAP2] / M2;
     } else {
-        g1 = 0.5 * 0.5 * a.hslash * (sd[SD_G1] / M) / a.f;
-        g2 = 0.5 * a.hslash * (sd[SD_G2] / M) / a.f;
-        x1 = (sd[SD_X1] / M) / a.f; x2 = (sd[SD_X2] / M) / a.f;
+        g1 = 0.5 * 0.5 * hslash * (sd[SD_G1] / M) / f;
+        g2 = 0.5 * hslash * (sd[SD_G2] / M) / f;
+        x1 = (sd[SD_X1] / M) / f; x2 = (sd[SD_X2] / M) / f;
         lap2m = sd[SD_LAP2] / M;
     }
     const double ar = sd[SD_PHI_R] / M, ai = sd[SD_PHI_I] / M, br = sd[SD_QPC_R] / M, bi = sd[SD_QPC_I] / M;
     const double pi = 0.5 * (ar * bi + ai * br);
-    const double ep_psi = a.nu4 * (si[SI_QLAP2PSI] / M2) - a.nu * (si[SI_PLAPQ] / M2) + a.mu * (si[SI_PQ] / M2);
-    const double chi_phi = -0.5 * a.nu4w * (se[SE_WV6PHI] / M2) / a.kappa2 - 0.5 * a.nuw * lap2m / a.kappa2 -
-                           0.5 * a.muw * (sd[SD_GRAD2] / M) / a.kappa2;
-    const double ep_phi = -a.nu4w * lap2m - a.nuw * (sd[SD_GRAD2] / M) - a.muw * (sd[SD_PHI2] / M);
+    const double ep_psi = nu4 * (si[SI_QLAP2PSI] / M2) - nu * (si[SI_PLAPQ] / M2) + mu * (si[SI_PQ] / M2);
+    const double chi_phi = -0.5 * nu4w * (se[SE_WV6PHI] / M2) / kappa2 - 0.5 * nuw * lap2m / kappa2 -
+                           0.5 * muw * (sd[SD_GRAD2] / M) / kappa2;
+    const double ep_phi = -nu4w * lap2m - nuw * (sd[SD_GRAD2] / M) - muw * (sd[SD_PHI2] / M);
     sc[NIWQG_S_GAMMA1] = g1; sc[NIWQG_S_GAMMA2] = g2; sc[NIWQG_S_XI1] = x1; sc[NIWQG_S_XI2] = x2; sc[NIWQG_S_PI] = pi;
     if (a.stage == 0) {
         sc[NIWQG_S_EP_PSI] = ep_psi; sc[NIWQG_S_CHI_PHI] = chi_phi; sc[NIWQG_S_EP_PHI] = ep_phi;
@@ -646,8 +655,7 @@ __global__ void k_budget(BudgetArgs a) {
 
 static BudgetArgs budget_args(niwqg_handle* h, int stage) {
     BudgetArgs b{};
-    b.stage = stage; b.M = h->Mg; b.f = h->p.f; b.hslash = h->hslash; b.kappa2 = h->kappa2; b.dt = h->p.dt;
-    b.nu4 = h->p.nu4; b.nu = h->p.nu; b.mu = h->p.mu; b.nu4w = h->p.nu4w; b.nuw = h->p.nuw; b.muw = h->p.muw;
+    b.stage = stage; b.M = h->Mg; b.dt = h->p.dt; b.mcoef = h->mcoef;
     b.sumsD = h->sumsD; b.sumsE = h->sumsE; b.sumsI = h->sumsI; b.scal = h->scal; b.stagev = h->stagev;
     b.spec_budget = (h->flags & MF_SPEC_BUDGET) ? 1 : 0;
     return b;
@@ -735,7 +743,7 @@ static int wave_fields(niwqg_handle* h, bool want_phi, bool grad, bool lap) {
 static int invert_family(niwqg_handle* h, bool keep_qwh = true) {
     InvertArgs ia{};
     ia.g = h->g;
-    ia.flags = h->flags; ia.f = h->p.f; ia.qh = h->qh[h->cq]; ia.filtr = h->filtr;
+    ia.flags = h->flags; ia.qh = h->qh[h->cq]; ia.filtr = h->filtr;
     ia.filtr_sym = (h->p.use_filter || !h->p.dealias) ? 1 : 0;
     ia.ph = h->ph; ia.qs = h->qs;
     if (h->flags & MF_WAVE_PV) {
@@ -747,7 +755,7 @@ static int invert_family(niwqg_handle* h, bool keep_qwh = true) {
     }
     if (h->flags & MF_YBJ) ia.uvgen = h->uv;
     ia.partials = (h->flags & MF_YBJ) ? nullptr : h->part;
-    { PROF(PK_SPEC); k_spec_invert<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(ia); }
+    { PROF(PK_SPEC); k_spec_invert<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(ia, h->mcoef); }
     CK(cudaGetLastError());
     h->launches++;
     if (ia.partials) FIN(SI_COUNT, h->sumsI);   // ep_psi sums of the state the next stage starts from
@@ -764,7 +772,7 @@ static int invert_family(niwqg_handle* h, bool keep_qwh = true) {
 static PhysArgs phys_args(niwqg_handle* h, int extra_flags) {
     PhysArgs pa{};
     pa.npts = h->npts; pa.flags = h->flags | extra_flags;
-    pa.nu4w = h->p.nu4w; pa.nuw = h->p.nuw; pa.muw = h->p.muw;
+    pa.mcoef = h->mcoef;
     pa.uv = h->uv; pa.qs = h->qs; pa.phi = h->phi; pa.phix = h->phix; pa.phiy = h->phiy;
     pa.lapphi = h->lapphi; pa.lap2phi = h->lap2phi; pa.uvq = h->uvq;
     pa.P1 = h->P1; pa.P2 = h->P2; pa.partials = h->part;
@@ -894,14 +902,14 @@ static int step_family(niwqg_handle* h) {
             }
             if (ybj) {
                 sa.sums_here = 0;
-                { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream))); }
+                { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream, h->pm_p))); }
                 h->launches++;
             } else {
                 // two lighter kernels: q equation, then phi equation + the stage's spectral budget sums
                 sa.do_q = 1; sa.do_phi = 0; sa.sums_here = 0;
-                { PROF(PK_SPEC); CK((launch_spec_stage<true, false>(sa, pw_grid(h), h->stream))); }
+                { PROF(PK_SPEC); CK((launch_spec_stage<true, false>(sa, pw_grid(h), h->stream, h->pm_q))); }
                 sa.do_q = 0; sa.do_phi = 1; sa.sums_here = 1;
-                { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream))); }
+                { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream, h->pm_p))); }
                 h->launches += 2;
             }
             if (st == 1) { h->cq = nq; h->cp = np; }
@@ -914,7 +922,7 @@ static int step_family(niwqg_handle* h) {
             FIN(SD_COUNT, h->sumsD);
             FFT(h->P1, h->P1, false, PRO_NONE, h->B);
             sa.do_phi = 0; sa.sums_here = 1;
-            { PROF(PK_SPEC); CK((launch_spec_stage<true, false>(sa, pw_grid(h), h->stream))); }
+            { PROF(PK_SPEC); CK((launch_spec_stage<true, false>(sa, pw_grid(h), h->stream, h->pm_q))); }
             if (st == 1) h->cq = nq;
             int r = ql_wave_velocity(h);
             if (r) return r;
@@ -923,7 +931,7 @@ static int step_family(niwqg_handle* h) {
             CK(cudaGetLastError());
             FFT(h->P2, h->P2, false, PRO_NONE, h->B);
             sa.do_q = 0; sa.do_phi = 1; sa.sums_here = 0;
-            { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream))); }
+            { PROF(PK_SPEC); CK((launch_spec_stage<false, true>(sa, pw_grid(h), h->stream, h->pm_p))); }
             h->launches += 4;
             if (st == 1) h->cp = np;
         }
@@ -995,14 +1003,20 @@ static int step_qg(niwqg_handle* h) {
         sa.y0c = h->chh[oc]; sa.yc = h->chh[nc]; sa.y1c = h->y1c; sa.F0c = h->F0c; sa.Fabc = h->Fabc;
         sa.tq = h->tq; sa.tc = h->tc; sa.filtr = h->filtr; sa.partials = h->part;
         sa.nu4c = h->p.nu4c;
-        { PROF(PK_SPEC); k_qg_stage<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(sa); }
+        {
+            PROF(PK_SPEC);
+            const dim3 g = pw_grid(h);
+            if (h->pm_q && h->pm_c) k_qg_stage<true, true><<<g, NIWQG_PW_THREADS, 0, h->stream>>>(sa);
+            else if (h->pm_q) k_qg_stage<true, false><<<g, NIWQG_PW_THREADS, 0, h->stream>>>(sa);
+            else if (h->pm_c) k_qg_stage<false, true><<<g, NIWQG_PW_THREADS, 0, h->stream>>>(sa);
+            else k_qg_stage<false, false><<<g, NIWQG_PW_THREADS, 0, h->stream>>>(sa);
+        }
         CK(cudaGetLastError());
         h->launches++;
         if (st == 1) { h->cq = nq; h->cc = nc; }
         FIN(QE_COUNT, h->sumsE);
         QgBudgetArgs ba{};
-        ba.stage = st; ba.M = h->Mg; ba.dt = h->p.dt; ba.nu4 = h->p.nu4; ba.nu = h->p.nu; ba.mu = h->p.mu;
-        ba.nu4c = h->p.nu4c; ba.muc = h->p.muc; ba.ps = ps ? 1 : 0;
+        ba.stage = st; ba.M = h->Mg; ba.dt = h->p.dt; ba.mcoef = h->mcoef; ba.ps = ps ? 1 : 0;
         ba.sumsE = h->sumsE; ba.scal = h->scal; ba.stagev = h->stagev;
         { PROF(PK_SMALL); k_qg_budget<<<h->B, 32, 0, h->stream>>>(ba); }
         CK(cudaGetLastError());
@@ -1222,10 +1236,15 @@ static int create_impl(niwqg_handle* h) {
         const double kmid = h->dk * N / 8.0;
         h->jscale = exp2(rint(log2(1.0 / (kmid * kmid))));
     }
+    h->kappa2m.assign(h->B, 0.0);
+    h->hslashm.assign(h->B, 0.0);
     if (!h->qg) {
-        const double kappa = p.m * p.f / p.N;     // Kernel.py:121-125
-        h->kappa2 = kappa * kappa;
-        h->hslash = p.f / h->kappa2;
+        for (int b = 0; b < h->B; ++b) {
+            const niwqg_member_params& c = h->mp[b];
+            const double kappa = c.m * c.f / c.N;     // Kernel.py:121-125
+            h->kappa2m[b] = kappa * kappa;
+            h->hslashm[b] = c.f / h->kappa2m[b];
+        }
     }
     switch (p.model) {
         case NIWQG_MODEL_COUPLED: h->flags = MF_WAVE_PV | MF_FIX00 | MF_SPEC_BUDGET; break;
@@ -1234,7 +1253,8 @@ static int create_impl(niwqg_handle* h) {
         case NIWQG_MODEL_QL: h->flags = MF_WAVE_PV | MF_QL_ADV; break;
         default: h->flags = 0;
     }
-    if (!h->qg && p.nu4w != 0.0) h->flags |= MF_HAS_LAP2;
+    for (int b = 0; b < h->B; ++b)
+        if (!h->qg && h->mp[b].nu4w != 0.0) h->flags |= MF_HAS_LAP2;
     const size_t B = h->B, cb = sizeof(cd);
     const size_t fsz = B * h->npts * cb, ssz = B * h->nspec * cb, tsz = h->nspec * cb;
     // twiddles
@@ -1258,35 +1278,76 @@ static int create_impl(niwqg_handle* h) {
         CK(cudaMemcpyAsync(h->twc, tw.data(), tw.size() * cb, cudaMemcpyHostToDevice, h->stream));
         CK(cudaStreamSynchronize(h->stream));
     }
-    // tables
-    auto alloc_tables = [&](TableSet& t) -> int {
-        DA(t.E, tsz); DA(t.E2, tsz); DA(t.Q, tsz); DA(t.f0, tsz); DA(t.fab, tsz); DA(t.fc, tsz);
-        return 0;
-    };
+    {   // per-member coefficients of the kernels (k_spec_invert, k_phys_rhs, k_budget, k_qg_budget, set_phi's Pw)
+        std::vector<double> mc((size_t)B * MC_COUNT);
+        for (size_t b = 0; b < B; ++b) {
+            const niwqg_member_params& c = h->mp[b];
+            double* r = &mc[b * MC_COUNT];
+            r[MC_F] = c.f; r[MC_HSLASH] = h->hslashm[b]; r[MC_KAPPA2] = h->kappa2m[b];
+            r[MC_NU4] = c.nu4; r[MC_NU] = c.nu; r[MC_MU] = c.mu; r[MC_NU4W] = c.nu4w; r[MC_NUW] = c.nuw; r[MC_MUW] = c.muw;
+            r[MC_NU4C] = c.nu4c; r[MC_MUC] = c.muc;
+            r[MC_PW_SEED] = h->qg ? 0.0 : 0.25 / h->Mg / h->kappa2m[b];
+        }
+        DA(h->mcoef, mc.size() * sizeof(double));
+        CK(cudaMemcpyAsync(h->mcoef, mc.data(), mc.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+    }
+    // tables: one set per equation, or one per member when the members' coefficients of that equation differ
     DA(h->filtr, h->nspec * sizeof(double));
     InitArgs ia{};
-    ia.g = h->g; ia.N = N; ia.nk = h->nk; ia.half = h->qg ? 1 : 0; ia.dk = h->dk; ia.dt = p.dt; ia.dx = h->dx; ia.U = p.U;
+    ia.g = h->g; ia.N = N; ia.nk = h->nk; ia.half = h->qg ? 1 : 0; ia.dk = h->dk; ia.dt = p.dt; ia.dx = h->dx;
     ia.use_filter = p.use_filter; ia.dealias = p.dealias;
     bool filtr_done = false;
-    if (p.model != NIWQG_MODEL_YBJ) {
-        if (alloc_tables(h->tq)) return -2;
-        ia.re_a4 = p.nu4; ia.re_a2 = p.nu; ia.re_a0 = p.mu; ia.im_wv2 = 0.0; ia.beta = h->qg ? p.beta : 0.0;
-        ia.t = h->tq; ia.filtr = h->filtr; filtr_done = true;
-        k_init_tables<<<NIWQG_PW_BLOCKS, NIWQG_PW_THREADS, 0, h->stream>>>(ia);
+    // row[IC_*] of member b for one equation (eq 0: q, 1: phi, 2: passive scalar c)
+    auto eq_row = [&](int eq, int b, double* r) {
+        const niwqg_member_params& c = h->mp[b];
+        if (eq == 0) { r[IC_RE_A4] = c.nu4; r[IC_RE_A2] = c.nu; r[IC_RE_A0] = c.mu; r[IC_IM_WV2] = 0.0; r[IC_BETA] = h->qg ? c.beta : 0.0; r[IC_U] = c.U; }
+        else if (eq == 1) { r[IC_RE_A4] = c.nu4w; r[IC_RE_A2] = c.nuw; r[IC_RE_A0] = c.muw; r[IC_IM_WV2] = 0.5 * c.f / h->kappa2m[b]; r[IC_BETA] = 0.0; r[IC_U] = c.U; }
+        else { r[IC_RE_A4] = c.nu4c; r[IC_RE_A2] = c.nuc; r[IC_RE_A0] = c.muc; r[IC_IM_WV2] = 0.0; r[IC_BETA] = 0.0; r[IC_U] = 0.0; }   // QGModel.py:452
+    };
+    // equal in every member: the keywords of the equation (niwqg_member_params), not the derived rows
+    auto eq_shared = [&](int eq) {
+        for (int b = 1; b < h->B; ++b) {
+            const niwqg_member_params &c = h->mp[b], &c0 = h->mp[0];
+            const bool same = eq == 0 ? (c.U == c0.U && c.nu4 == c0.nu4 && c.nu == c0.nu && c.mu == c0.mu && (!h->qg || c.beta == c0.beta))
+                            : eq == 1 ? (c.U == c0.U && c.f == c0.f && c.N == c0.N && c.m == c0.m && c.nu4w == c0.nu4w &&
+                                         c.nuw == c0.nuw && c.muw == c0.muw)
+                                      : (c.nu4c == c0.nu4c && c.nuc == c0.nuc && c.muc == c0.muc);
+            if (!same) return false;
+        }
+        return true;
+    };
+    auto init_eq = [&](int eq, TableSet& t, bool& pm) -> int {
+        pm = !eq_shared(eq);
+        const size_t tb = (pm ? B : 1) * tsz;
+        DA(t.E, tb); DA(t.E2, tb); DA(t.Q, tb); DA(t.f0, tb); DA(t.fab, tb); DA(t.fc, tb);
+        ia.t = t;
+        ia.filtr = filtr_done ? nullptr : h->filtr;
+        filtr_done = true;
+        double r[IC_COUNT];
+        eq_row(eq, 0, r);
+        ia.re_a4 = r[IC_RE_A4]; ia.re_a2 = r[IC_RE_A2]; ia.re_a0 = r[IC_RE_A0]; ia.im_wv2 = r[IC_IM_WV2];
+        ia.beta = r[IC_BETA]; ia.U = r[IC_U];
+        ia.mc = nullptr;
+        if (pm) {   // every member's row, filled in one launch (member = blockIdx.y)
+            std::vector<double> rows(B * IC_COUNT);
+            for (size_t b = 0; b < B; ++b) eq_row(eq, (int)b, &rows[b * IC_COUNT]);
+            double* d = nullptr;
+            DA(d, rows.size() * sizeof(double));
+            CK(cudaMemcpyAsync(d, rows.data(), rows.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            ia.mc = d;
+        }
+        k_init_tables<<<dim3(NIWQG_PW_BLOCKS, pm ? h->B : 1), NIWQG_PW_THREADS, 0, h->stream>>>(ia);
         CK(cudaGetLastError());
-    }
-    if (!h->qg) {
-        if (alloc_tables(h->tp)) return -2;
-        ia.re_a4 = p.nu4w; ia.re_a2 = p.nuw; ia.re_a0 = p.muw; ia.im_wv2 = 0.5 * p.f / h->kappa2; ia.beta = 0.0;
-        ia.t = h->tp; ia.filtr = filtr_done ? nullptr : h->filtr;
-        k_init_tables<<<NIWQG_PW_BLOCKS, NIWQG_PW_THREADS, 0, h->stream>>>(ia);
-        CK(cudaGetLastError());
-    } else if (p.passive_scalar) {
-        if (alloc_tables(h->tc)) return -2;
-        ia.re_a4 = p.nu4c; ia.re_a2 = p.nuc; ia.re_a0 = p.muc; ia.im_wv2 = 0.0; ia.beta = 0.0; ia.U = 0.0;   // QGModel.py:452
-        ia.t = h->tc; ia.filtr = nullptr;
-        k_init_tables<<<NIWQG_PW_BLOCKS, NIWQG_PW_THREADS, 0, h->stream>>>(ia);
-        CK(cudaGetLastError());
+        return 0;
+    };
+    {
+        int r = 0;
+        if (p.model != NIWQG_MODEL_YBJ) r = init_eq(0, h->tq, h->pm_q);
+        if (!r && !h->qg) r = init_eq(1, h->tp, h->pm_p);
+        else if (!r && p.passive_scalar) r = init_eq(2, h->tc, h->pm_c);
+        if (r) return r;
     }
     // state
     DA(h->qh[0], ssz); DA(h->ph, ssz); DA(h->uv, fsz); DA(h->qs, fsz);
@@ -1353,7 +1414,18 @@ static int create_impl(niwqg_handle* h) {
     return 0;
 }
 
-int niwqg_create(const niwqg_params* p, niwqg_handle** out) {
+// the coefficient fields of p, as member parameters
+static niwqg_member_params member_of(const niwqg_params& p) {
+    niwqg_member_params c{};
+    c.struct_size = sizeof(niwqg_member_params);
+    c.U = p.U; c.f = p.f; c.N = p.N; c.m = p.m; c.nu = p.nu; c.nu4 = p.nu4; c.mu = p.mu;
+    c.nuw = p.nuw; c.nu4w = p.nu4w; c.muw = p.muw; c.beta = p.beta; c.nu4c = p.nu4c; c.nuc = p.nuc; c.muc = p.muc;
+    return c;
+}
+
+int niwqg_create(const niwqg_params* p, niwqg_handle** out) { return niwqg_create_ensemble(p, nullptr, out); }
+
+int niwqg_create_ensemble(const niwqg_params* p, const niwqg_member_params* members, niwqg_handle** out) {
     if (!p || !out) { g_create_error = "null argument"; return -1; }
     *out = nullptr;
     if (p->struct_size != sizeof(niwqg_params)) {
@@ -1375,8 +1447,23 @@ int niwqg_create(const niwqg_params* p, niwqg_handle** out) {
         g_create_error = "no CUDA device: niwqg_b200 has no CPU fallback";
         return -3;
     }
+    if (members)
+        for (int b = 0; b < p->batch; ++b)
+            if (members[b].struct_size != sizeof(niwqg_member_params)) {
+                g_create_error = "niwqg_member_params.struct_size does not match this library (binding built against another header)";
+                return -1;
+            }
     niwqg_handle* h = new niwqg_handle();
     h->p = *p;
+    h->mp.assign(p->batch, member_of(*p));
+    if (members) {
+        for (int b = 0; b < p->batch; ++b) h->mp[b] = members[b];
+        // the batch-1 paths (split / fused step, jacobians) and everything shared read p: member 0's coefficients
+        const niwqg_member_params& c = members[0];
+        h->p.U = c.U; h->p.f = c.f; h->p.N = c.N; h->p.m = c.m; h->p.nu = c.nu; h->p.nu4 = c.nu4; h->p.mu = c.mu;
+        h->p.nuw = c.nuw; h->p.nu4w = c.nu4w; h->p.muw = c.muw; h->p.beta = c.beta;
+        h->p.nu4c = c.nu4c; h->p.nuc = c.nuc; h->p.muc = c.muc;
+    }
     int r = create_impl(h);
     if (r) { g_create_error = h->err; niwqg_destroy(h); return r; }
     *out = h;
@@ -1455,8 +1542,11 @@ static int ke_qg_family(niwqg_handle* h) {   // 0.5*spec_var(wv*ph) (Kernel.py:6
     return 0;
 }
 
-__global__ void k_set_scalar_from_sum(double* scal, int slot, const double* sums, int K, int idx, double factor) {
+// scal[m][slot] = factor * sums[m][idx]; mfactor != null: the member's factor mfactor[m * MC_COUNT] instead
+__global__ void k_set_scalar_from_sum(double* scal, int slot, const double* sums, int K, int idx, double factor,
+                                      const double* mfactor = nullptr) {
     const int m = blockIdx.x;
+    if (mfactor) factor = mfactor[(size_t)m * MC_COUNT];
     if (threadIdx.x == 0) scal[(size_t)m * NIWQG_S_COUNT + slot] = factor * sums[(size_t)m * K + idx];
 }
 
@@ -1548,7 +1638,7 @@ static int seed_phi(niwqg_handle* h) {
     int r = pe_niw_refresh(h, h->sumsX);
     if (r) return r;
     const double M = h->Mg;
-    k_set_scalar_from_sum<<<h->B, 32, 0, h->stream>>>(h->scal, NIWQG_S_PW, h->sumsX, 1, 0, 0.25 / M / h->kappa2);
+    k_set_scalar_from_sum<<<h->B, 32, 0, h->stream>>>(h->scal, NIWQG_S_PW, h->sumsX, 1, 0, 0.0, h->mcoef + MC_PW_SEED);
     CK(cudaGetLastError());
     k_phi2_sum<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(h->phi, h->npts, h->part);
     CK(cudaGetLastError());
@@ -1780,7 +1870,7 @@ int niwqg_status(niwqg_handle* h, double* out) {
     for (int m = 0; m < B; ++m) {
         out[m * 4 + 0] = 0.5 * p_ke[(size_t)m * SS_COUNT + SS_KE] / M2;
         out[m * 4 + 1] = 0.5 * p_kw[m] / M;
-        out[m * 4 + 2] = 0.25 * p_pw[m] / M / h->kappa2;
+        out[m * 4 + 2] = 0.25 * p_pw[m] / M / h->kappa2m[m];
         out[m * 4 + 3] = p_cfl[m] * h->p.dt / h->dx;
     }
     return 0;
@@ -1826,13 +1916,14 @@ int niwqg_diagnostics(niwqg_handle* h, double* out) {
             o[NIWQG_S_CVAR] = ps ? sc[(size_t)m * NIWQG_S_COUNT + NIWQG_S_CVAR] : 0.0;
             o[NIWQG_S_KE_QG] = 0.5 * s[QS_KE] / M2;
             o[NIWQG_S_ENS] = 0.5 * sq[m] / M;
-            o[NIWQG_S_EP_PSI] = h->p.nu4 * s[QS_QLAP2PSI] / M2 - h->p.nu * s[QS_PLAPQ] / M2 + h->p.mu * s[QS_PQ] / M2;
-            o[NIWQG_S_CHI_Q] = -h->p.nu4 * s[QS_CHIQ] / M2;
+            const niwqg_member_params& p = h->mp[m];
+            o[NIWQG_S_EP_PSI] = p.nu4 * s[QS_QLAP2PSI] / M2 - p.nu * s[QS_PLAPQ] / M2 + p.mu * s[QS_PQ] / M2;
+            o[NIWQG_S_CHI_Q] = -p.nu4 * s[QS_CHIQ] / M2;
             if (ps) {
                 const double C2 = s[QS_C2] / M2, gradC2 = s[QS_GRADC2] / M2, lapc2 = s[QS_LAPC2] / M2, lap2clapc = s[QS_LAP2CLAPC] / M2;
                 o[NIWQG_S_C2] = C2; o[NIWQG_S_GRADC2] = gradC2; o[NIWQG_S_GAMMA_C] = gam[m];
-                o[NIWQG_S_EP_C] = -2 * h->p.nu4c * lapc2 - 2 * h->p.nu * gradC2 - 2 * h->p.muc * C2;          // QGModel.py:595-598
-                o[NIWQG_S_CHI_C] = 2 * h->p.nu4c * lap2clapc - 2 * h->p.nu * lapc2 - 2 * h->p.muc * gradC2;  // QGModel.py:600-604
+                o[NIWQG_S_EP_C] = -2 * p.nu4c * lapc2 - 2 * p.nu * gradC2 - 2 * p.muc * C2;          // QGModel.py:595-598
+                o[NIWQG_S_CHI_C] = 2 * p.nu4c * lap2clapc - 2 * p.nu * lapc2 - 2 * p.muc * gradC2;  // QGModel.py:600-604
             }
         }
         return 0;
@@ -1876,8 +1967,9 @@ int niwqg_diagnostics(niwqg_handle* h, double* out) {
     if (r) return r;
     CK(cudaMemcpyAsync(p_sg, h->sumsE, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    const niwqg_params& p = h->p;
     for (int m = 0; m < B; ++m) {
+        const niwqg_member_params& p = h->mp[m];
+        const double hslash = h->hslashm[m], kappa2 = h->kappa2m[m];
         double* o = out + (size_t)m * NIWQG_S_COUNT;
         const double* D = &p_sd[(size_t)m * SD_COUNT];
         const double* S = &p_ss[(size_t)m * SS_COUNT];
@@ -1885,8 +1977,8 @@ int niwqg_diagnostics(niwqg_handle* h, double* out) {
         o[NIWQG_S_KE] = p_sc[(size_t)m * NIWQG_S_COUNT + NIWQG_S_KE];
         o[NIWQG_S_PW] = p_sc[(size_t)m * NIWQG_S_COUNT + NIWQG_S_PW];
         o[NIWQG_S_KW] = p_sc[(size_t)m * NIWQG_S_COUNT + NIWQG_S_KW];
-        o[NIWQG_S_GAMMA1] = 0.5 * 0.5 * h->hslash * (D[SD_G1] / M) / p.f;
-        o[NIWQG_S_GAMMA2] = 0.5 * h->hslash * (D[SD_G2] / M) / p.f;
+        o[NIWQG_S_GAMMA1] = 0.5 * 0.5 * hslash * (D[SD_G1] / M) / p.f;
+        o[NIWQG_S_GAMMA2] = 0.5 * hslash * (D[SD_G2] / M) / p.f;
         o[NIWQG_S_XI1] = (D[SD_X1] / M) / p.f;
         o[NIWQG_S_XI2] = (D[SD_X2] / M) / p.f;
         const double ar = D[SD_PHI_R] / M, ai = D[SD_PHI_I] / M, br = D[SD_QPC_R] / M, bi = D[SD_QPC_I] / M;
@@ -1897,7 +1989,7 @@ int niwqg_diagnostics(niwqg_handle* h, double* out) {
         o[NIWQG_S_CKE_NIW] = 0.5 * (ar * ar + ai * ai);
         o[NIWQG_S_IKE_NIW] = o[NIWQG_S_KE_NIW] - o[NIWQG_S_CKE_NIW];
         const double grad2 = p_sg[m] / M;     // refreshed phix, phiy
-        o[NIWQG_S_PE_NIW] = 0.25 * grad2 / h->kappa2;
+        o[NIWQG_S_PE_NIW] = 0.25 * grad2 / kappa2;
         const double* c3 = &p_s3[(size_t)m * 3];
         o[NIWQG_S_CONC] = (c3[0] / M) / sqrt(c3[1] / M) / sqrt(c3[2] / M);
         o[NIWQG_S_SKEW] = (D[SD_QP3] / M) / pow(D[SD_QP2] / M, 1.5);
@@ -1908,8 +2000,8 @@ int niwqg_diagnostics(niwqg_handle* h, double* out) {
         else
             o[NIWQG_S_EP_PSI] = p.nu4 * S[SS_QLAP2PSI] / M2 - p.nu * S[SS_PLAPQ] / M2 + p.mu * S[SS_PQ] / M2;
         o[NIWQG_S_CHI_Q] = -p.nu4 * S[SS_CHIQ] / M2;
-        o[NIWQG_S_CHI_PHI] = -0.5 * p.nu4w * (S[SS_WV6PHI] / M2) / h->kappa2 - 0.5 * p.nuw * lap2m / h->kappa2 -
-                             0.5 * p.muw * grad2 / h->kappa2;
+        o[NIWQG_S_CHI_PHI] = -0.5 * p.nu4w * (S[SS_WV6PHI] / M2) / kappa2 - 0.5 * p.nuw * lap2m / kappa2 -
+                             0.5 * p.muw * grad2 / kappa2;
         if (h->flags & MF_WAVE_PV) {
             o[NIWQG_S_KE_QG_Q] = 0.5 * S[SS_KEQ] / M2;
             o[NIWQG_S_KE_QG_W] = 0.5 * S[SS_KEW] / M2;
@@ -1988,24 +2080,24 @@ static int get_field_impl(niwqg_handle* h, int field, int member, void* dst, siz
         case NIWQG_F_QWH: src = h->qwh ? h->qwh + so : nullptr; break;
         case NIWQG_F_CH: src = h->chh[h->cc] ? h->chh[h->cc] + so : nullptr; break;
         case NIWQG_F_FILTR: src = h->filtr; break;
-        case NIWQG_F_EXPCH: src = h->tq.E; break;
-        case NIWQG_F_EXPCH_H: src = h->tq.E2; break;
-        case NIWQG_F_QHCOEF: src = h->tq.Q; break;
-        case NIWQG_F_F0: src = h->tq.f0; break;
-        case NIWQG_F_FAB: src = h->tq.fab; break;
-        case NIWQG_F_FC: src = h->tq.fc; break;
-        case NIWQG_F_EXPCHW: src = h->tp.E; break;
-        case NIWQG_F_EXPCH_HW: src = h->tp.E2; break;
-        case NIWQG_F_QHWCOEF: src = h->tp.Q; break;
-        case NIWQG_F_F0W: src = h->tp.f0; break;
-        case NIWQG_F_FABW: src = h->tp.fab; break;
-        case NIWQG_F_FCW: src = h->tp.fc; break;
-        case NIWQG_F_EXPCHC: src = h->tc.E; break;
-        case NIWQG_F_EXPCH_HC: src = h->tc.E2; break;
-        case NIWQG_F_QHCCOEF: src = h->tc.Q; break;
-        case NIWQG_F_F0C: src = h->tc.f0; break;
-        case NIWQG_F_FABC: src = h->tc.fab; break;
-        case NIWQG_F_FCC: src = h->tc.fc; break;
+        case NIWQG_F_EXPCH: src = h->tq.E + (h->pm_q ? so : 0); break;
+        case NIWQG_F_EXPCH_H: src = h->tq.E2 + (h->pm_q ? so : 0); break;
+        case NIWQG_F_QHCOEF: src = h->tq.Q + (h->pm_q ? so : 0); break;
+        case NIWQG_F_F0: src = h->tq.f0 + (h->pm_q ? so : 0); break;
+        case NIWQG_F_FAB: src = h->tq.fab + (h->pm_q ? so : 0); break;
+        case NIWQG_F_FC: src = h->tq.fc + (h->pm_q ? so : 0); break;
+        case NIWQG_F_EXPCHW: src = h->tp.E + (h->pm_p ? so : 0); break;
+        case NIWQG_F_EXPCH_HW: src = h->tp.E2 + (h->pm_p ? so : 0); break;
+        case NIWQG_F_QHWCOEF: src = h->tp.Q + (h->pm_p ? so : 0); break;
+        case NIWQG_F_F0W: src = h->tp.f0 + (h->pm_p ? so : 0); break;
+        case NIWQG_F_FABW: src = h->tp.fab + (h->pm_p ? so : 0); break;
+        case NIWQG_F_FCW: src = h->tp.fc + (h->pm_p ? so : 0); break;
+        case NIWQG_F_EXPCHC: src = h->tc.E + (h->pm_c ? so : 0); break;
+        case NIWQG_F_EXPCH_HC: src = h->tc.E2 + (h->pm_c ? so : 0); break;
+        case NIWQG_F_QHCCOEF: src = h->tc.Q + (h->pm_c ? so : 0); break;
+        case NIWQG_F_F0C: src = h->tc.f0 + (h->pm_c ? so : 0); break;
+        case NIWQG_F_FABC: src = h->tc.fab + (h->pm_c ? so : 0); break;
+        case NIWQG_F_FCC: src = h->tc.fc + (h->pm_c ? so : 0); break;
         default: h->err = "get_field: unknown field"; return -1;
     }
     if (r) return r;
