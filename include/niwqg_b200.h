@@ -228,6 +228,32 @@ int niwqg_ipc_import(niwqg_handle* h, const char* all_ranks, size_t bytes_per_ra
 /* switch back to the NCCL all-to-all exchange (all ranks must agree, e.g. after one of them failed to import) */
 int niwqg_ipc_disable(niwqg_handle* h);
 
+/* Lagrangian particles (drifters, DESIGN.md section 3.4).  A particle is a point (x, y) in metres in the frame of the
+ * model's grid (values at the cell centres x_i = (i + 1/2) dx, physical arrays [iy][ix]), stored unwrapped in fp64;
+ * velocities are interpolated periodically with the tensor-product 4-point (cubic) Lagrange stencil.  Every step
+ * advances the particles by classical RK4 whose four stages read the model's own ETDRK4 stage fields: stage 1 the
+ * state at t_n, stages 2 and 3 the states a and b at t_n + dt/2, stage 4 the state c at t_n + dt, each as the model
+ * carries it (YBJ: its frozen u, v and the phi of t_n, which stays stale through the stages).  The velocity is
+ * U + u_psi (the member's mean flow and the packed uv buffer); with waves, plus the wave velocity at the level where
+ * the vertical factor is 1, u_w + i v_w = exp(-i f t) phi (the member's f; inertial loops are clockwise for f > 0).
+ * In the Coupled and QL models u_psi is already the Lagrangian-mean flow, so waves=1 gives drifter-like loops but
+ * counts the O(a^2) Stokes drift twice.  The wave phase uses a device clock set here and advanced by dt every step.
+ * Particles only read the model: fields, scalars and diagnostics are bit for bit those of a run without them.
+ * Single-GPU handles only: a slab handle (nranks > 1) returns an error from every call below but the count.
+ *
+ * niwqg_particles_set: xy = batch x count x 2 doubles (host, or device when on_device), all finite; t = the clock;
+ * waves = 1 adds the wave velocity (models with phi only).  count = 0 removes the particles.  Replaces any particles
+ * already set.  Seeding or removing drops the captured step graphs, which the next steps capture again.
+ * niwqg_particles_count: particles per member (0: none).
+ * niwqg_particles_get: xy = the batch x count x 2 positions, *t = the clock (either may be NULL).
+ * niwqg_particles_sample: field = NIWQG_F_Q, NIWQG_F_U, NIWQG_F_V (out: batch x count doubles) or NIWQG_F_PHI (out:
+ * batch x count complex), interpolated at the current positions with the same stencil, from exactly what
+ * niwqg_get_field returns.  Changes no state. */
+int niwqg_particles_set(niwqg_handle* h, const double* xy, int count, double t, int waves, int on_device);
+int niwqg_particles_count(const niwqg_handle* h);
+int niwqg_particles_get(niwqg_handle* h, double* xy, double* t);
+int niwqg_particles_sample(niwqg_handle* h, int field, double* out);
+
 int niwqg_sync(niwqg_handle* h);
 /* CUDA-event timing on the handle's stream: elapsed ms of `nsteps` steps */
 int niwqg_time_steps(niwqg_handle* h, int nsteps, float* ms);

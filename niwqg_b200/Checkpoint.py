@@ -7,6 +7,8 @@ A checkpoint is a directory::
     <SLOT>.npy         one per state slot, whole grid in natural order with a leading member axis:
                        (batch, nx, nx), or (batch, nx, nx/2+1) for the QG half spectrum
     diagnostics.npz    the 'value' array of every diagnostic that has one
+    PARTICLES.npy      only for a model with Lagrangian particles: their unwrapped positions, (batch, P, 2); the
+                       ``particles`` entry of checkpoint.json holds P, the particle clock and ``waves``
 
 Which buffers make up the state is decided by the CUDA library (niwqg_state_slots); this module only moves them
 between the device and the files.  Fields are streamed one member at a time, so the host never holds more than one
@@ -31,6 +33,7 @@ FORMAT = "niwqg_b200-checkpoint"
 VERSION = 1
 META = "checkpoint.json"
 DIAGNOSTICS = "diagnostics.npz"
+PARTICLES = "PARTICLES"
 STATUS_ATTRS = ("ke", "kew", "pew", "cfl")
 
 
@@ -120,7 +123,7 @@ def _step(io, fn):
         raise err if err is not None else RuntimeError("writing the checkpoint failed on another rank")
 
 
-def write(path, meta, io, diagnostics=None):
+def write(path, meta, io, diagnostics=None, arrays=None):
     """Write the state behind ``io`` and the host-side ``meta`` (a JSON-able dict) as the checkpoint ``path``.
 
     ``path`` must not exist, be an empty directory or hold a checkpoint: any other directory is refused before anything
@@ -129,7 +132,7 @@ def write(path, meta, io, diagnostics=None):
     it was.  Replacing a directory takes two renames (``path`` -> ``.<name>.old``, ``.<name>.partial`` -> ``path``);
     if the process dies between them, ``locate`` finds the previous checkpoint under ``.<name>.old``.  In a slab run
     every rank calls this; rank 0 creates the files and does the replacing, and an error on any rank is raised on all
-    of them."""
+    of them.  ``arrays``: {name: array} written by rank 0 as ``<name>.npy`` beside the slots."""
     path = os.path.abspath(path)
     tmp, old = _aside(path, ".partial"), _aside(path, ".old")
     slots = io.slots()
@@ -161,6 +164,8 @@ def write(path, meta, io, diagnostics=None):
                     carry=[float(v) for v in io.get_carry()])
         if diagnostics:
             np.savez(os.path.join(tmp, DIAGNOSTICS), **diagnostics)
+        for name, a in (arrays or {}).items():
+            np.save(_file(tmp, name), a)
         with open(os.path.join(tmp, META), "w") as f:
             json.dump(full, f, indent=1)
             f.flush()
@@ -281,7 +286,13 @@ def save(model, path, dist=None):
     meta = dict(model=_class_name(type(model)), params=_keywords(model, model._checkpoint_params),
                 run=_keywords(model, model._checkpoint_run), t=model.t, tc=model.tc, status=status)
     diags = {k: d["value"] for k, d in model.diagnostics.items() if "value" in d}
-    write(path, meta, _io(model, dist), diags)
+    arrays = {}
+    ps = model._particles_state()
+    if ps is not None:
+        xy, t, waves = ps
+        meta["particles"] = dict(count=int(xy.shape[1]), t=t, waves=bool(waves))
+        arrays[PARTICLES] = xy
+    write(path, meta, _io(model, dist), diags, arrays)
 
 
 def load(model, path, dist=None, changed=()):
@@ -304,6 +315,7 @@ def load(model, path, dist=None, changed=()):
         raise ValueError("checkpoint %s does not match the model: %s" % (path, ", ".join(diffs)))
     io = _io(model, dist)
     check(path, meta, io)
+    xy = _check_particles(path, meta, model)
     values = read(path, meta, io)
     model.t, model.tc = meta["t"], meta["tc"]
     for name, d in model.diagnostics.items():
@@ -311,6 +323,11 @@ def load(model, path, dist=None, changed=()):
             d["value"] = values[name]
         else:
             d.pop("value", None)
+    if xy is not None:
+        pm = meta["particles"]
+        model._set_particles_state(xy, pm["t"], pm["waves"])
+    elif model._particles_state() is not None:
+        model.set_particles(None)       # the saved run had none
     for k in STATUS_ATTRS:
         v = meta["status"].get(k)
         v = None if v is None else (np.array(v) if isinstance(v, list) else v)
@@ -320,6 +337,25 @@ def load(model, path, dist=None, changed=()):
             model.__dict__.pop(k, None)
         else:
             setattr(model, k, v)
+
+
+def _check_particles(path, meta, model):
+    """The saved particle positions (batch, P, 2), or None when the checkpoint has no particles.  Reads and checks them
+    before anything on the model changes."""
+    pm = meta.get("particles")
+    if pm is None:
+        return None
+    if model._h.nranks > 1:
+        raise NotImplementedError("checkpoint %s has Lagrangian particles: a slab-decomposed model cannot carry them"
+                                  % path)
+    fn = _file(path, PARTICLES)
+    if not os.path.exists(fn):
+        raise FileNotFoundError("checkpoint %s: missing %s" % (path, os.path.basename(fn)))
+    xy = np.load(fn)
+    if xy.dtype != np.float64 or xy.shape != (model.batch, pm["count"], 2):
+        raise ValueError("checkpoint %s: %s is %s %s, expected float64 %s"
+                         % (path, os.path.basename(fn), xy.dtype, xy.shape, (model.batch, pm["count"], 2)))
+    return xy
 
 
 def from_checkpoint(cls, path, dist=None, **overrides):

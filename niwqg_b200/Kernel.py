@@ -12,6 +12,7 @@ from numpy import pi
 
 from . import _native as nat
 from . import Checkpoint
+from .Particles import Particles
 from .Diagnostics import add_diagnostic, increment_diagnostics, get_diagnostic, describe_diagnostics  # noqa: F401
 from .Saving import initialize_save_snapshots, save_setup, save_snapshots, save_diagnostics
 
@@ -68,7 +69,7 @@ def _wv2i(self):
     return out
 
 
-class Kernel(object):
+class Kernel(Particles):
     """Doubly periodic single-vertical-mode NIW + barotropic QG pseudo-spectral kernel.
 
     Parameters are those of niwqg/Kernel.py:70-98 (SI units), plus

@@ -7,12 +7,13 @@ from numpy import pi
 
 from . import _native as nat
 from . import Checkpoint
+from .Particles import Particles
 from .Kernel import _DeviceField, _Scalar, _LazyGrid, _wv2i
 from .Diagnostics import add_diagnostic, increment_diagnostics
 from .Saving import initialize_save_snapshots, save_setup, save_snapshots, save_diagnostics
 
 
-class Model(object):
+class Model(Particles):
     """Parameters: niwqg/QGModel.py:65-91, plus ``batch`` and ``device``.  With batch > 1, each of U, beta, nu, nu4,
     mu, nu4c, nuc, muc may be a sequence of batch values, one per member; nx, L, dt, use_filter, dealias and
     passive_scalar are common to all members."""

@@ -47,7 +47,8 @@ EXPORTS = ["niwqg_create", "niwqg_destroy", "niwqg_last_error", "niwqg_set_q", "
            "niwqg_launch_count", "niwqg_stream", "niwqg_profile", "niwqg_nccl_unique_id", "niwqg_ic",
            "niwqg_get_field_async", "niwqg_wait_transfers", "niwqg_stage_q", "niwqg_stage_phi",
            "niwqg_ipc_export", "niwqg_ipc_import", "niwqg_ipc_disable", "niwqg_state_slots", "niwqg_set_field",
-           "niwqg_carry_count", "niwqg_get_carry", "niwqg_set_carry", "niwqg_create_ensemble"]
+           "niwqg_carry_count", "niwqg_get_carry", "niwqg_set_carry", "niwqg_create_ensemble",
+           "niwqg_particles_set", "niwqg_particles_count", "niwqg_particles_get", "niwqg_particles_sample"]
 
 
 class Params(C.Structure):
@@ -138,6 +139,10 @@ def load():
     lib.niwqg_carry_count.argtypes = [vp]
     lib.niwqg_get_carry.argtypes = [vp, vp]
     lib.niwqg_set_carry.argtypes = [vp, vp]
+    lib.niwqg_particles_set.argtypes = [vp, vp, ip, C.c_double, ip, ip]
+    lib.niwqg_particles_count.argtypes = [vp]
+    lib.niwqg_particles_get.argtypes = [vp, vp, vp]
+    lib.niwqg_particles_sample.argtypes = [vp, ip, vp]
     _lib = lib
     return lib
 
@@ -193,6 +198,29 @@ def slab_owner(N, nranks, kx):
         return 0, h
     m = N - kx
     return m // h, h + m % h
+
+
+# fields niwqg_particles_sample interpolates, by the name Model.sample_particles takes
+PARTICLE_FIELDS = {"q": "Q", "u": "U", "v": "V", "phi": "PHI"}
+
+
+def particle_positions(xy, batch):
+    """Validate the positions given to set_particles: (P, 2) seeds every member, (batch, P, 2) each member its own.
+    Returns a C-contiguous float64 (batch, P, 2) array.  ValueError for another shape or a non-finite value."""
+    a = np.asarray(xy)
+    if a.dtype.kind not in "iuf":
+        raise ValueError("particle positions must be real numbers, got dtype %s" % a.dtype)
+    a = a.astype(np.float64)
+    if a.ndim == 2 and a.shape[1] == 2:
+        a = np.broadcast_to(a[None], (batch,) + a.shape)
+    if a.ndim != 3 or a.shape[0] != batch or a.shape[2] != 2 or a.shape[1] == 0:
+        raise ValueError("particle positions must have shape (P, 2) or (batch=%d, P, 2) with P >= 1, got %s"
+                         % (batch, np.shape(xy)))
+    if a.shape[1] > 2 ** 31 - 1:
+        raise ValueError("at most 2**31 - 1 particles per member")
+    if not np.all(np.isfinite(a)):
+        raise ValueError("particle positions must be finite")
+    return np.ascontiguousarray(a)
 
 
 class Handle(object):
@@ -434,6 +462,33 @@ class Handle(object):
         if a.size != self.lib.niwqg_carry_count(self.h):
             raise ValueError("expected %d carry values, got %d" % (self.lib.niwqg_carry_count(self.h), a.size))
         self._ck(self.lib.niwqg_set_carry(self.h, a.ctypes.data))
+
+    # -- Lagrangian particles ---------------------------------------------
+    def particles_set(self, xy, t, waves):
+        """xy: (batch, P, 2) float64 as particle_positions returns it, or None to remove the particles."""
+        if xy is None:
+            self._ck(self.lib.niwqg_particles_set(self.h, None, 0, float(t), 0, 0))
+            return
+        self._ck(self.lib.niwqg_particles_set(self.h, xy.ctypes.data, xy.shape[1], float(t), int(bool(waves)), 0))
+
+    def particles_count(self):
+        return int(self.lib.niwqg_particles_count(self.h))
+
+    def particles(self):
+        """(positions (batch, P, 2), clock), or (None, None) without particles."""
+        n = self.particles_count()
+        if n == 0:
+            return None, None
+        xy = np.empty((self.B, n, 2))
+        t = np.zeros(1)
+        self._ck(self.lib.niwqg_particles_get(self.h, xy.ctypes.data, t.ctypes.data))
+        return xy, float(t[0])
+
+    def particles_sample(self, name):
+        n = self.particles_count()
+        out = np.empty((self.B, n), np.complex128 if name == "PHI" else np.float64)
+        self._ck(self.lib.niwqg_particles_sample(self.h, F[name], out.ctypes.data))
+        return out
 
     def field_to_device(self, name, member, ptr, nbytes):
         self._ck(self.lib.niwqg_get_field(self.h, F[name], member, C.c_void_p(ptr), nbytes, 1))

@@ -76,8 +76,9 @@ struct TableSet { cd *E, *E2, *Q, *f0, *fab, *fc; };
 
 // Per-member coefficients the kernels read by value of blockIdx.y: mcoef[member][MC_COUNT] (equal rows when the
 // members share their parameters).  MC_PW_SEED = 0.25 / (N^2 kappa2), the Pw of set_phi per unit grad^2 sum.
+// MC_U: the uniform mean flow U (the -ikU of the linear operator), which Lagrangian particles add to u.
 enum { MC_F = 0, MC_HSLASH, MC_KAPPA2, MC_NU4, MC_NU, MC_MU, MC_NU4W, MC_NUW, MC_MUW, MC_NU4C, MC_MUC, MC_PW_SEED,
-       MC_COUNT };
+       MC_U, MC_COUNT };
 
 // coefficients of one equation's exponent c (see InitArgs), per member for k_init_tables
 enum { IC_RE_A4 = 0, IC_RE_A2, IC_RE_A0, IC_IM_WV2, IC_BETA, IC_U, IC_COUNT };

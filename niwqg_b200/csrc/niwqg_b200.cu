@@ -19,6 +19,7 @@
 #include "kernels_fused.cuh"
 #include "kernels_qg.cuh"
 #include "kernels_ic.cuh"
+#include "kernels_particles.cuh"
 
 static std::string g_create_error;
 
@@ -138,6 +139,11 @@ struct niwqg_handle {
     std::vector<ProfRec> prof_recs;
     std::vector<cudaEvent_t> prof_pool;
     size_t prof_used = 0;
+    // Lagrangian particles (kernels_particles.cuh): np per member, none when 0.  One allocation: x_n, the stage position
+    // and the RK4 accumulator ([B][np] double2 each), then the particle clock (2 doubles)
+    int np = 0;
+    bool pwaves = false;
+    double2* pbuf = nullptr;
 };
 
 enum { PK_FFT_ROW = 0, PK_FFT_COL, PK_PHYS, PK_SPEC, PK_SMALL, PK_COMM, PK_FFT_P, PK_FFT_ROWLD, PK_FFT_ROWLD2, PK_COUNT };
@@ -787,6 +793,39 @@ static int ql_wave_velocity(niwqg_handle* h) {   // uq, vq from the current qh (
     return 0;
 }
 
+// ---------------------------------------------------------------------------
+// Lagrangian particles: one RK4 stage wherever the model's uv (and phi) hold the fields of ETDRK4 stage `st`
+// ---------------------------------------------------------------------------
+static PartArgs particle_args(const niwqg_handle* h) {
+    PartArgs a{};
+    a.xn = h->pbuf; a.xs = h->pbuf + (size_t)h->B * h->np; a.acc = h->pbuf + 2 * (size_t)h->B * h->np;
+    a.clk = (double*)(h->pbuf + 3 * (size_t)h->B * h->np);
+    a.mcoef = h->mcoef; a.npts = h->npts; a.P = h->np; a.N = h->N;
+    a.dshift = h->deintC > 1 ? 1 : 0;               // deintC is 1 or 2 (split path)
+    a.dM = h->deintC > 1 ? h->deintM : h->N;
+    a.L = h->p.L; a.dx = h->dx; a.dt = h->p.dt;
+    return a;
+}
+static dim3 particle_grid(const niwqg_handle* h) { return dim3((unsigned)((h->np + 127) / 128), h->B); }
+
+static int particles_stage(niwqg_handle* h, int st) {
+    if (!h->np) return 0;
+    PartArgs a = particle_args(h);
+    a.uv = h->uv; a.phi = h->pwaves ? h->phi : nullptr;
+    const dim3 g = particle_grid(h);
+    cudaStream_t s = h->stream;
+#define NIWQG_PSTAGE(S)                                                        \
+    case S:                                                                    \
+        if (h->pwaves) k_particles<S, true><<<g, 128, 0, s>>>(a);              \
+        else k_particles<S, false><<<g, 128, 0, s>>>(a);                       \
+        break;
+    switch (st) { NIWQG_PSTAGE(1) NIWQG_PSTAGE(2) NIWQG_PSTAGE(3) NIWQG_PSTAGE(4) }
+#undef NIWQG_PSTAGE
+    CK(cudaGetLastError());
+    h->launches++;
+    return 0;
+}
+
 // Coupled / UnCoupled step on the split transform path with the fused spectral kernels (kernels_fused.cuh): the
 // forward transforms stop after their M-point column transforms, the kernel that consumes the spectrum does the radix
 // combine itself; the kernels that produce a spectrum emit the radix stage of its inverse transforms.
@@ -798,6 +837,7 @@ static int step_family_fused_n(niwqg_handle* h) {
     const int grid = WAVE_CTAS;     // persistent grid of the fused kernels
     int r;
     for (int st = 1; st <= 4; ++st) {
+        if ((r = particles_stage(h, st))) return r;
         PhysArgs pa = phys_args(h, MF_P1_BY_LOADER);
         { PROF(PK_PHYS); k_phys_rhs<<<pw_grid(h), NIWQG_PW_THREADS, 0, h->stream>>>(pa); }
         CK(cudaGetLastError());
@@ -873,6 +913,7 @@ static int step_family(niwqg_handle* h) {
     const int oq = h->cq, op = h->cp;          // y0 buffers
     const int nq = ybj ? oq : 1 - oq, np = 1 - op;
     for (int st = 1; st <= 4; ++st) {
+        if (int rp = particles_stage(h, st)) return rp;
         if (ybj) {   // _calc_grad_phi from the stage's phih (YBJModel.py:135-139); phi stays stale (F7)
             const cd* cur = (st == 1) ? h->phih[op] : h->phih[np];
             const FftJob jobs[2] = {FftJob{cur, h->phix, true, PRO_IK}, FftJob{cur, h->phiy, true, PRO_IL}};
@@ -984,6 +1025,7 @@ static int step_qg(niwqg_handle* h) {
         const cd* cur = (st == 1) ? h->qh[oq] : h->qh[nq];
         int r = qg_expand_and_invert(h, cur);
         if (r) return r;
+        if ((r = particles_stage(h, st))) return r;
         const cd* ccur = nullptr;
         if (ps) {
             ccur = (st == 1) ? h->chh[oc] : h->chh[nc];
@@ -1186,6 +1228,7 @@ int niwqg_destroy(niwqg_handle* h) {
         if (h->pre_free[w]) cudaEventDestroy(h->pre_free[w]);
     }
     if (h->pin) cudaFreeHost(h->pin);
+    if (h->pbuf) cudaFree(h->pbuf);
     if (h->ev0) cudaEventDestroy(h->ev0);
     if (h->ev1) cudaEventDestroy(h->ev1);
     if (h->stream) cudaStreamDestroy(h->stream);
@@ -1287,6 +1330,7 @@ static int create_impl(niwqg_handle* h) {
             r[MC_NU4] = c.nu4; r[MC_NU] = c.nu; r[MC_MU] = c.mu; r[MC_NU4W] = c.nu4w; r[MC_NUW] = c.nuw; r[MC_MUW] = c.muw;
             r[MC_NU4C] = c.nu4c; r[MC_MUC] = c.muc;
             r[MC_PW_SEED] = h->qg ? 0.0 : 0.25 / h->Mg / h->kappa2m[b];
+            r[MC_U] = c.U;
         }
         DA(h->mcoef, mc.size() * sizeof(double));
         CK(cudaMemcpyAsync(h->mcoef, mc.data(), mc.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
@@ -2333,6 +2377,103 @@ int niwqg_jacobian(niwqg_handle* h, int which, void* out) {
             CK(cudaMemcpyAsync(out, h->P1, c, cudaMemcpyDeviceToHost, h->stream));
         }
     }
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+
+// ---- Lagrangian particles (kernels_particles.cuh, DESIGN.md section 3.4)
+static const char* const PARTICLES_SLAB =
+    "particles: not available on a slab handle (nranks > 1): particles would have to migrate between ranks";
+
+int niwqg_particles_set(niwqg_handle* h, const double* xy, int count, double t, int waves, int on_device) {
+    if (h->nranks > 1) { h->err = PARTICLES_SLAB; return -1; }
+    if (count < 0) { h->err = "particles_set: count must be >= 0"; return -1; }
+    if (count > 0 && !xy) { h->err = "particles_set: null positions"; return -1; }
+    if (waves && !h->phi) { h->err = "particles_set: waves=1 needs a model with a wave field phi (not QGModel)"; return -1; }
+    if (!std::isfinite(t)) { h->err = "particles_set: the clock t must be finite"; return -1; }
+    CK(cudaSetDevice(h->p.device));
+    const size_t n = (size_t)h->B * count;           // particles over all members
+    std::vector<double> host;
+    if (on_device && count > 0) {                    // checked on the host like any other input
+        host.resize(2 * n);
+        CK(cudaMemcpy(host.data(), xy, 2 * n * sizeof(double), cudaMemcpyDeviceToHost));
+        xy = host.data();
+    }
+    for (size_t i = 0; i < 2 * n; ++i)
+        if (!std::isfinite(xy[i])) { h->err = "particles_set: positions must be finite"; return -1; }
+    const size_t bytes = 3 * n * sizeof(double2) + 2 * sizeof(double);
+    if (count > 0) {
+        size_t fr = 0, tot = 0;
+        CK(cudaMemGetInfo(&fr, &tot));
+        if (bytes > fr) {
+            char buf[256];
+            snprintf(buf, sizeof buf, "particles_set: %zu particles need %zu bytes of device memory, %zu are free", n, bytes, fr);
+            h->err = buf;
+            return -1;
+        }
+    }
+    // the step graphs captured the particle launches (or their absence): drop them, the next steps capture anew
+    CK(cudaStreamSynchronize(h->stream));
+    for (auto& g : h->graphs)
+        if (g.exec) { CK(cudaGraphExecDestroy(g.exec)); g = niwqg_handle::StepGraph{}; }
+    if (h->pbuf) { CK(cudaFree(h->pbuf)); h->pbuf = nullptr; }
+    h->np = 0;
+    h->pwaves = false;
+    if (count == 0) return 0;
+    CK(cudaMalloc((void**)&h->pbuf, bytes));
+    h->np = count;
+    h->pwaves = waves != 0;
+    const double clk[2] = {t, t};
+    CK(cudaMemcpyAsync(h->pbuf, xy, n * sizeof(double2), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync((double*)(h->pbuf + 3 * n), clk, sizeof clk, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int niwqg_particles_count(const niwqg_handle* h) { return h->np; }
+
+int niwqg_particles_get(niwqg_handle* h, double* xy, double* t) {
+    if (h->nranks > 1) { h->err = PARTICLES_SLAB; return -1; }
+    if (!h->np) { h->err = "particles_get: the model has no particles"; return -1; }
+    CK(cudaSetDevice(h->p.device));
+    const size_t n = (size_t)h->B * h->np;
+    if (xy) CK(cudaMemcpyAsync(xy, h->pbuf, n * sizeof(double2), cudaMemcpyDeviceToHost, h->stream));
+    if (t) CK(cudaMemcpyAsync(t, (const double*)(h->pbuf + 3 * n), sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int niwqg_particles_sample(niwqg_handle* h, int field, double* out) {
+    if (h->nranks > 1) { h->err = PARTICLES_SLAB; return -1; }
+    if (!h->np) { h->err = "particles_sample: the model has no particles"; return -1; }
+    CK(cudaSetDevice(h->p.device));
+    PartArgs a = particle_args(h);
+    const size_t n = (size_t)h->B * h->np;
+    // the result goes to the stage-position and accumulator arrays: every step writes them before it reads them
+    double2* dout = a.xs;
+    const dim3 g = particle_grid(h);
+    if (field == NIWQG_F_PHI) {
+        if (!h->phi) { h->err = "particles_sample: the model has no wave field phi"; return -1; }
+        k_particles_sample<cd><<<g, 128, 0, h->stream>>>(a, h->phi, dout);
+    } else {
+        const cd* src = nullptr;
+        int which = 0;
+        switch (field) {   // what niwqg_get_field returns: the same extraction into scratch, for every member
+            case NIWQG_F_Q: src = h->qs; which = 0; break;
+            case NIWQG_F_U: src = h->uv; which = 0; break;
+            case NIWQG_F_V: src = h->uv; which = 1; break;
+            default: h->err = "particles_sample: field must be Q, U, V or PHI"; return -1;
+        }
+        k_extract_real<<<NIWQG_PW_BLOCKS, NIWQG_PW_THREADS, 0, h->stream>>>(src, h->rscratch, (size_t)h->B * h->npts, which);
+        CK(cudaGetLastError());
+        h->launches++;
+        k_particles_sample<double><<<g, 128, 0, h->stream>>>(a, h->rscratch, (double*)dout);
+    }
+    CK(cudaGetLastError());
+    h->launches++;
+    const size_t w = (field == NIWQG_F_PHI) ? 2 : 1;
+    CK(cudaMemcpyAsync(out, dout, n * w * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return 0;
 }
